@@ -7,6 +7,8 @@ synthetic clips (config 1's shape tiled to a batch, SURVEY.md 8(d)): CLIPS_PER_G
 44.1 kHz, n_fft 2048, hop 512, Blackman (the AnalyserNode window), u8 output.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          this repo's CUDA path
+  python bench.py ... --dump-outputs DIR                        also writes a seeded sample of the last timed step's
+                                                               output to DIR/spectrogram.npy (float32, rank 0)
   python bench.py --impl reference ...                          the CPU arm (oracle port, all host threads)
   torchrun ... bench.py --gpus N ...                            one rank per GPU, clips sharded, no collective
                                                                on the data path (shards are independent)
@@ -154,10 +156,10 @@ def cpu_arm(x, steps: int, warmup: int, threads: int = 0) -> dict:
     times = []
     for _ in range(max(steps, 1)):
         t0 = time.perf_counter()
-        cref.stft_batch(x, cfg, threads)
+        y = cref.stft_batch(x, cfg, threads)
         times.append(time.perf_counter() - t0)
     dt = sum(times) / len(times)
-    return {"value": frames / dt, "unit": "frames/s", "cores": cores, "kind": "port",
+    return {"value": frames / dt, "unit": "frames/s", "cores": cores, "kind": "port", "out": y,
             "sample": f"{n_clips} clips x 10 s x 44.1 kHz ({frames} frames) per step, {len(times)} steps, "
                       f"oracle/analyser_ref.c float32, {cores} thread{'s' if cores != 1 else ''}",
             "ms_per_step": dt * 1e3, "ms_min": min(times) * 1e3, "ms_max": max(times) * 1e3, "frames": frames}
@@ -206,6 +208,9 @@ def run_reference(args) -> None:
     n_clips = args.clips_per_gpu                  # the GPU arm's batch, clip for clip (same `config`)
     x = synth_clips_cpu(n_clips)
     r = cpu_arm(x, args.steps, args.warmup)
+    if args.dump_outputs:
+        import torch
+        dump_outputs(args.dump_outputs, torch.from_numpy(r["out"]))
     line = {
         "impl": "reference", "metric": "stft_frames_per_s", "value": r["value"], "unit": "frames/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
@@ -245,6 +250,22 @@ def synth_clips_gpu(torch, n_clips: int, first_clip: int, device):
         ph = 0.37 * torch.arange(first_clip + c0, first_clip + c1, dtype=torch.float64, device=device)
         x[c0:c1] = (0.5 * torch.sin(base[None, :] + ph[:, None])).to(torch.float32)
     return x
+
+
+DUMP_ROWS = 12288            # 48 MB as float32: under the 64 MB a dump may take
+
+
+def dump_outputs(dirname: str, out, rows: int = DUMP_ROWS, seed: int = 0) -> None:
+    """Writes `rows` output rows of `out` (all of them if it has fewer; [clip, frame] pairs drawn without replacement by a
+    fixed seed, in flattened order) as float32 to dirname/spectrogram.npy, so that two builds run with the same arguments
+    compare row for row."""
+    import numpy as np
+    import torch
+    flat = out.reshape(-1, out.shape[-1])
+    idx = np.sort(np.random.default_rng(seed).choice(flat.shape[0], min(rows, flat.shape[0]), replace=False))
+    sample = flat[torch.from_numpy(idx).to(flat.device)].float().cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "spectrogram.npy"), sample)
 
 
 def bind_near_gpu(index: int) -> str:
@@ -462,6 +483,8 @@ def run_gpu(args) -> None:
     ms = max_over_ranks(ms_local, dev)
     total_frames = sum_over_ranks(frames, dev)
     value = total_frames / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)     # `out` still holds the last timed step's result
 
     # ---- parity spot check of what was just timed (rank 0, first clip) against the oracle
     parity = None
@@ -631,7 +654,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE configs 2-5 block (N = 1 only anyway)")
     ap.add_argument("--quick-configs", action="store_true", help="smaller config 2 / 4 / 5 workloads (development)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's output to "
+                                                          "DIR/spectrogram.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,4 +1,5 @@
-"""Host-side logic that needs no GPU: options mapping, sharding, the multi-process bench plumbing."""
+"""Host-side logic that needs no GPU: options mapping, sharding, the multi-process bench plumbing, bench.py's output dump
+(the GPU arm's under ``-m gpu``)."""
 import os
 import subprocess
 import sys
@@ -79,9 +80,9 @@ print("ok", rank)
     assert r.stdout.count("ok") == 2
 
 
-def test_reference_arm_prints_the_contract_line():
+def test_reference_arm_prints_the_contract_line(tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
-                        "--clips-per-gpu", "8"],
+                        "--clips-per-gpu", "8", "--dump-outputs", str(tmp_path / "dump")],
                        capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     import json
@@ -90,3 +91,45 @@ def test_reference_arm_prints_the_contract_line():
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["config"]["n_fft"] == 2048
     assert line["config"]["clips_per_gpu"] == 8      # the CPU arm runs the GPU arm's batch, clip for clip
+    # 8 clips x 858 frames is below the dump's row budget: every row of the timed step's output, in order
+    import bench
+    from oracle import analyser_oracle as O
+    from oracle import cref
+    dump = np.load(tmp_path / "dump" / "spectrogram.npy")
+    want = cref.stft_batch(bench.synth_clips_cpu(8), O.Config(window=O.WINDOW_BLACKMAN, output=O.OUT_U8))
+    assert dump.dtype == np.float32 and np.array_equal(dump, want.reshape(-1, 1024))
+
+
+@pytest.mark.gpu
+def test_gpu_arm_times_the_given_steps_and_dumps_the_same_outputs_every_run(tmp_path):
+    import json
+    from oracle import analyser_oracle as O
+    from _tol import assert_bytes_close
+    lines, dumps = [], []
+    for run in range(2):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "1", "--clips-per-gpu", "8",
+                            "--e2e-clips", "0", "--no-cpu-baseline", "--no-configs", "--dump-outputs", str(tmp_path / str(run))],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        lines.append(json.loads(r.stdout.strip().splitlines()[-1]))
+        dumps.append(np.load(tmp_path / str(run) / "spectrogram.npy"))
+    assert lines[0]["steps"] == 3 and lines[0]["gpu_launches"] == 3      # one launch per step
+    assert dumps[0].dtype == np.float32 and dumps[0].shape == (8 * 858, 1024)   # every row: 8 clips are below the budget
+    assert np.array_equal(dumps[0], dumps[1])
+    import bench
+    ref = O.spectrogram(bench.synth_clips_cpu(1, first_clip=7)[0], O.Config())[0]
+    assert_bytes_close(dumps[0][7 * 858:], ref)
+
+
+def test_dump_is_a_fixed_sample_of_whole_rows_within_64_mb(tmp_path):
+    import torch
+    import bench
+    n = 40000                                    # rows: more than the dump keeps; each row holds its own index
+    out = torch.arange(n, dtype=torch.int32)[:, None].expand(n, 1024).reshape(40, 1000, 1024)
+    bench.dump_outputs(str(tmp_path / "a"), out)
+    bench.dump_outputs(str(tmp_path / "b"), out)
+    a, b = np.load(tmp_path / "a" / "spectrogram.npy"), np.load(tmp_path / "b" / "spectrogram.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_ROWS, 1024) and a.nbytes <= 64 << 20
+    assert np.array_equal(a, b)
+    rows = a[:, 0]
+    assert np.all(a == rows[:, None]) and np.all(np.diff(rows) > 0) and rows[0] >= 0 and rows[-1] < n
