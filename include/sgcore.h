@@ -214,8 +214,14 @@ int sg_stream_info(const sg_stream* s, int* channels, int* hop, int* bins, int* 
  * whatever channels arrive to mono ([SPEC] AnalyserNode: "as if channelCount 1, channelCountMode max,
  * channelInterpretation speakers").  Built here for uncompressed PCM (RIFF/WAVE or raw interleaved
  * samples): sample-format conversion and the speakers down-mix run on the GPU, so 16-bit audio crosses
- * PCIe at 2 bytes per sample.  Compressed formats and sample-rate conversion are NOT built (the browser's
- * decoder/resampler are implementation-defined; sample_rate is carried through unchanged). */
+ * PCIe at 2 bytes per sample.  Compressed formats are NOT decoded.  decodeAudioData also resamples to the
+ * context's rate; the *_resampled calls below do that on the GPU, fused with the conversion, with one fixed
+ * filter: rational polyphase resampling equal to scipy.signal.resample_poly(x, up, down) with its default
+ * Kaiser(beta 5) window (up/down = out_rate/in_rate reduced, half = 10*max(up, down), taps h[m] =
+ * c sinc(c(m - half)) kaiser(m), c = 1/max(up, down), sum 1, times up; samples outside the clip are 0),
+ * accumulated in float32.  Rates are integers in [3000, 768000] Hz and the reduced max(up, down) must be
+ * <= 16384, else SG_ERR_INDEX_SIZE.  Equal rates take the plain ingest, bit for bit.  The other calls
+ * carry sample_rate through unchanged. */
 typedef enum sg_pcm_format {
   SG_PCM_U8 = 0,  /* unsigned 8 bit:            (v - 128) / 128                                 */
   SG_PCM_S16 = 1, /* little-endian signed 16:   v / 32768                                       */
@@ -234,7 +240,7 @@ typedef enum sg_pcm_layout {
 typedef struct sg_pcm_info {
   int32_t format;      /* sg_pcm_format                                                          */
   int32_t channels;    /* 1..32 interleaved channels                                             */
-  int32_t sample_rate; /* Hz, informational                                                      */
+  int32_t sample_rate; /* Hz: the source rate of the *_resampled calls, informational elsewhere    */
   int64_t frames;      /* sample frames per clip (AudioBuffer.length)                            */
   int64_t data_offset; /* sg_wav_parse: byte offset of the first sample in the file; the ingest
                           calls take a pointer to the first sample and ignore this field         */
@@ -260,6 +266,18 @@ int sg_pcm_ingest_device(sg_engine* e, const void* pcm_dev, int64_t n_clips, con
  * what crosses PCIe; copies, ingest and frame kernels overlap chunk by chunk. */
 int sg_stft_pcm(sg_engine* e, const void* pcm, int64_t n_clips, const sg_pcm_info* info, int layout,
                 const sg_stft_config* cfg, void* out);
+/* frames after resampling `frames` from in_rate to out_rate: ceil(frames*up/down); <0 for invalid rates */
+int64_t sg_resample_num_frames(int64_t frames, int32_t in_rate, int32_t out_rate);
+/* sg_pcm_ingest, resampled from info->sample_rate to out_rate: out host [n_clips][planes][out_frames] */
+int sg_pcm_ingest_resampled(sg_engine* e, const void* pcm, int64_t n_clips, const sg_pcm_info* info, int layout,
+                            int32_t out_rate, float* out);
+/* same on device buffers, asynchronous; plane p of clip c at out_dev + (c*planes+p)*out_stride, out_stride >= out_frames */
+int sg_pcm_ingest_resampled_device(sg_engine* e, const void* pcm_dev, int64_t n_clips, const sg_pcm_info* info,
+                                   int layout, int32_t out_rate, float* out_dev, int64_t out_stride, void* cuda_stream);
+/* sg_stft_pcm with the planes resampled to out_rate before framing: out [n_clips][planes][frames(out_frames)][bins].
+ * Bit-identical to sg_pcm_ingest_resampled followed by sg_stft_batch on the planes. */
+int sg_stft_pcm_resampled(sg_engine* e, const void* pcm, int64_t n_clips, const sg_pcm_info* info, int layout,
+                          int32_t out_rate, const sg_stft_config* cfg, void* out);
 
 /* ------------------------------------------------------------------ sonogram ring + view --- */
 /* The reference's spectrogram history: a bins x rows ALPHA/UNSIGNED_BYTE texture, one byte row per

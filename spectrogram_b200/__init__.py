@@ -8,10 +8,10 @@ from ._lib import (ALIGN_ANALYSER, ALIGN_VALID, OUT_F32_DB, OUT_F32_MAG, OUT_RGB
                    WINDOW_CUSTOM, WINDOW_HANN, WINDOW_RECT, EngineError, IndexSizeError)
 from .analyser import AnalyserNode
 from .api import (AudioBuffer, Engine, Options, PinnedArray, SonogramRing, StreamBank, colormap_reference, default_engine, device_count,
-                  shard_bounds, spectrogram, spectrogram_multi, wav_info)
+                  resample_num_frames, shard_bounds, spectrogram, spectrogram_multi, wav_info)
 
 __all__ = [
-    "AnalyserNode", "AudioBuffer", "wav_info", "Engine", "Options", "PinnedArray", "StreamBank", "SonogramRing", "spectrogram", "spectrogram_multi", "colormap_reference",
+    "AnalyserNode", "AudioBuffer", "wav_info", "resample_num_frames", "Engine", "Options", "PinnedArray", "StreamBank", "SonogramRing", "spectrogram", "spectrogram_multi", "colormap_reference",
     "default_engine", "device_count", "shard_bounds", "IndexSizeError", "EngineError",
     "WINDOW_BLACKMAN", "WINDOW_HANN", "WINDOW_RECT", "WINDOW_CUSTOM",
     "OUT_U8", "OUT_F32_DB", "OUT_RGBA8", "OUT_F32_MAG", "ALIGN_VALID", "ALIGN_ANALYSER",

@@ -110,6 +110,13 @@ SIGNATURES = {
                                        C.c_int64, C.c_void_p]),
     "sg_stft_pcm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(PcmInfo), C.c_int, C.POINTER(StftConfig),
                               C.c_void_p]),
+    "sg_resample_num_frames": (C.c_int64, [C.c_int64, C.c_int32, C.c_int32]),
+    "sg_pcm_ingest_resampled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(PcmInfo), C.c_int, C.c_int32,
+                                          C.c_void_p]),
+    "sg_pcm_ingest_resampled_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(PcmInfo), C.c_int,
+                                                 C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
+    "sg_stft_pcm_resampled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(PcmInfo), C.c_int, C.c_int32,
+                                        C.POINTER(StftConfig), C.c_void_p]),
     "sg_ring_create": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "sg_ring_destroy": (C.c_int, [C.c_void_p]),
     "sg_ring_reset": (C.c_int, [C.c_void_p]),

@@ -94,6 +94,15 @@ def wav_info(file_bytes) -> "L.PcmInfo":
     return info
 
 
+def resample_num_frames(frames: int, in_rate: int, out_rate: int) -> int:
+    """Length after resampling ``frames`` sample frames from ``in_rate`` to ``out_rate`` Hz: ceil(frames*up/down)
+    (``sg_resample_num_frames``; host only).  IndexSizeError for rates the resampler does not take."""
+    n = int(L.load().sg_resample_num_frames(int(frames), int(in_rate), int(out_rate)))
+    if n < 0:
+        L.check(n)
+    return n
+
+
 class AudioBuffer:
     """What ``decodeAudioData`` hands the reference (util/util.js:10-12): planar float32 channels."""
 
@@ -202,39 +211,58 @@ class Engine:
 
     # -- PCM ingestion in front of the path (decodeAudioData for uncompressed PCM) -------------
     def decode_pcm(self, data, fmt: str = "s16", channels: int = 1, sample_rate: int = 48000, n_clips: int = 1,
-                   mix: bool = False) -> "AudioBuffer":
+                   mix: bool = False, context_rate: int | None = None) -> "AudioBuffer":
         """Interleaved samples (bytes-like or array) -> float32 planes on the GPU.  ``mix=True`` applies the
-        AnalyserNode's speakers down-mix to mono; otherwise every channel is a plane (AudioBuffer.getChannelData)."""
+        AnalyserNode's speakers down-mix to mono; otherwise every channel is a plane (AudioBuffer.getChannelData).
+        ``context_rate``: resample from ``sample_rate`` to this rate on the GPU, as decodeAudioData does for a
+        context running at that rate (``sg_pcm_ingest_resampled``)."""
         raw, info = _pcm_args(data, fmt, channels, sample_rate, n_clips)
         layout = L.PCM_MONO_MIX if mix else L.PCM_PLANAR
         planes = 1 if mix else channels
-        out = np.empty((n_clips, planes, info.frames), dtype=np.float32)
-        L.check(self._lib.sg_pcm_ingest(self.handle, raw.ctypes.data, n_clips, C.byref(info), layout, out.ctypes.data))
-        return AudioBuffer(out[0] if n_clips == 1 else out, sample_rate)
+        if context_rate is None:
+            out = np.empty((n_clips, planes, info.frames), dtype=np.float32)
+            L.check(self._lib.sg_pcm_ingest(self.handle, raw.ctypes.data, n_clips, C.byref(info), layout, out.ctypes.data))
+            return AudioBuffer(out[0] if n_clips == 1 else out, sample_rate)
+        length = resample_num_frames(info.frames, sample_rate, context_rate)
+        out = np.empty((n_clips, planes, length), dtype=np.float32)
+        L.check(self._lib.sg_pcm_ingest_resampled(self.handle, raw.ctypes.data, n_clips, C.byref(info), layout,
+                                                  int(context_rate), out.ctypes.data))
+        return AudioBuffer(out[0] if n_clips == 1 else out, context_rate)
 
-    def decode_audio_data(self, file_bytes, mix: bool = False) -> "AudioBuffer":
-        """``context.decodeAudioData(arrayBuffer)`` (util/util.js:9) for RIFF/WAVE files holding uncompressed PCM."""
+    def decode_audio_data(self, file_bytes, mix: bool = False, context_rate: int | None = None) -> "AudioBuffer":
+        """``context.decodeAudioData(arrayBuffer)`` (util/util.js:9) for RIFF/WAVE files holding uncompressed PCM.
+        ``context_rate``: the context's sample rate; the file's samples are resampled to it on the GPU."""
         buf = np.frombuffer(bytes(file_bytes) if not isinstance(file_bytes, (bytes, bytearray, memoryview)) else file_bytes,
                             dtype=np.uint8)
         info = wav_info(buf)
         body = buf[info.data_offset:info.data_offset + info.frames * info.channels * _PCM_BYTES[info.format]]
-        return self.decode_pcm(body, _PCM_FMT_OF[info.format], info.channels, info.sample_rate, 1, mix)
+        return self.decode_pcm(body, _PCM_FMT_OF[info.format], info.channels, info.sample_rate, 1, mix, context_rate)
 
     def spectrogram_pcm(self, data, fmt: str = "s16", channels: int = 1, n_clips: int = 1, mix: bool = True,
-                        opts: Options | None = None, **kw) -> np.ndarray:
+                        opts: Options | None = None, sample_rate: int | None = None, context_rate: int | None = None,
+                        **kw) -> np.ndarray:
         """Interleaved PCM bytes -> [clips, planes, frames, bins(,4)]: ingest fused in front of the batched path
-        (the raw bytes are what crosses PCIe)."""
+        (the raw bytes are what crosses PCIe).  ``context_rate``: resample from ``sample_rate`` (then required)
+        to this rate before framing, so bin k is k*context_rate/fftSize Hz whatever the source rate."""
         opts = opts or Options(**kw)
-        raw, info = _pcm_args(data, fmt, channels, 0, n_clips)
+        if context_rate is not None and sample_rate is None:
+            raise TypeError("context_rate needs the source sample_rate")
+        raw, info = _pcm_args(data, fmt, channels, sample_rate or 0, n_clips)
         cfg, _keep = opts.to_c()
-        frames = int(self._lib.sg_stft_num_frames(C.byref(cfg), info.frames))
+        length = info.frames if context_rate is None else resample_num_frames(info.frames, sample_rate, context_rate)
+        frames = int(self._lib.sg_stft_num_frames(C.byref(cfg), length))
         if frames < 0:
             L.check(L.SG_ERR_INDEX_SIZE)
         planes = 1 if mix else channels
         dt, shape = out_dtype_shape(cfg.output, n_clips * planes, frames, cfg.n_fft // 2)
         out = np.empty((n_clips, planes) + shape[1:], dtype=dt)
-        L.check(self._lib.sg_stft_pcm(self.handle, raw.ctypes.data, n_clips, C.byref(info),
-                                      L.PCM_MONO_MIX if mix else L.PCM_PLANAR, C.byref(cfg), out.ctypes.data))
+        layout = L.PCM_MONO_MIX if mix else L.PCM_PLANAR
+        if context_rate is None:
+            L.check(self._lib.sg_stft_pcm(self.handle, raw.ctypes.data, n_clips, C.byref(info), layout, C.byref(cfg),
+                                          out.ctypes.data))
+        else:
+            L.check(self._lib.sg_stft_pcm_resampled(self.handle, raw.ctypes.data, n_clips, C.byref(info), layout,
+                                                    int(context_rate), C.byref(cfg), out.ctypes.data))
         return out
 
     # -- batched path on device memory (pointers + a CUDA stream handle) ---------------------

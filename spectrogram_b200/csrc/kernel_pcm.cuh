@@ -45,6 +45,45 @@ template <> struct PcmFmt<kPcmS32> { static constexpr int kBytes = 4;
 template <> struct PcmFmt<kPcmF32> { static constexpr int kBytes = 4;
   static __device__ __forceinline__ float cvt(uint32_t v) { return __uint_as_float(v); } };
 
+// Stages bytes [b0, b0 + n) of src into s_q with 16-byte loads from the aligned-down address (bytes outside
+// [0, src_bytes) read as 0) and returns b0's offset inside the first staged word.  The caller synchronises.
+template <int THREADS>
+__device__ __forceinline__ int pcm_stage(uint4* s_q, const unsigned char* src, long long src_bytes, long long b0, int n) {
+  const int skew = (int)(((uintptr_t)src + (uintptr_t)b0) & 15);
+  const long long a0 = b0 - skew;                                 // 16-byte aligned (as an address), may be < 0
+  const int nq = (skew + n + 15) >> 4;
+  for (int i = threadIdx.x; i < nq; i += THREADS) {
+    const long long o = a0 + 16LL * i;
+    uint4 q;
+    if (o >= 0 && o + 16 <= src_bytes) {
+      q = __ldg(reinterpret_cast<const uint4*>(src + o));
+    } else {                                                      // first/last chunk of the buffer: byte by byte
+      uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+      for (int b = 0; b < 16; ++b)
+        if (o + b >= 0 && o + b < src_bytes) w[b >> 2] |= (uint32_t)src[o + b] << (8 * (b & 3));
+      q = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+    s_q[i] = q;
+  }
+  return skew;
+}
+
+// the sample starting at byte_off of the staged words: two adjacent 32-bit words and a funnel shift
+template <int FMT>
+__device__ __forceinline__ float pcm_pick(const uint32_t* __restrict__ sw, int byte_off) {
+  const int wi = byte_off >> 2;
+  return PcmFmt<FMT>::cvt(__funnelshift_r(sw[wi], sw[wi + 1], 8 * (byte_off & 3)));
+}
+
+// speakers down-mix of the sample frame at byte_off: w[0] x[0], then one FMA per further channel in channel order
+template <int FMT>
+__device__ __forceinline__ float pcm_mono(const uint32_t* __restrict__ sw, int byte_off, int channels, const PcmMix& m) {
+  float acc = m.w[0] * pcm_pick<FMT>(sw, byte_off);
+  for (int c = 1; c < channels; ++c) acc = fmaf(m.w[c], pcm_pick<FMT>(sw, byte_off + c * PcmFmt<FMT>::kBytes), acc);
+  return acc;
+}
+
 template <int FMT>
 __global__ void __launch_bounds__(kPcmThreads)
 pcm_ingest_kernel(const __grid_constant__ PcmGeom g, const __grid_constant__ PcmMix m) {
@@ -56,36 +95,14 @@ pcm_ingest_kernel(const __grid_constant__ PcmGeom g, const __grid_constant__ Pcm
   const int tf = (int)min((long long)g.tile_frames, g.frames - f0);
   const int bpf = g.channels * SB;
   const long long b0 = clip * g.clip_bytes + f0 * bpf;           // first byte of the tile, relative to src
-  const int skew = (int)(((uintptr_t)g.src + (uintptr_t)b0) & 15);
-  const long long a0 = b0 - skew;                                 // 16-byte aligned (as an address), may be < 0
-  const int nq = (skew + tf * bpf + 15) >> 4;
-  for (int i = threadIdx.x; i < nq; i += kPcmThreads) {
-    const long long o = a0 + 16LL * i;
-    uint4 q;
-    if (o >= 0 && o + 16 <= g.src_bytes) {
-      q = __ldg(reinterpret_cast<const uint4*>(g.src + o));
-    } else {                                                      // first/last chunk of the buffer: byte by byte
-      uint32_t w[4] = {0u, 0u, 0u, 0u};
-#pragma unroll
-      for (int b = 0; b < 16; ++b)
-        if (o + b >= 0 && o + b < g.src_bytes) w[b >> 2] |= (uint32_t)g.src[o + b] << (8 * (b & 3));
-      q = make_uint4(w[0], w[1], w[2], w[3]);
-    }
-    s_q[i] = q;
-  }
+  const int skew = pcm_stage<kPcmThreads>(s_q, g.src, g.src_bytes, b0, tf * bpf);
   __syncthreads();
   const uint32_t* __restrict__ sw = reinterpret_cast<const uint32_t*>(s_q);
-  auto sample = [&](int byte_off) {
-    const int wi = byte_off >> 2;
-    return PcmFmt<FMT>::cvt(__funnelshift_r(sw[wi], sw[wi + 1], 8 * (byte_off & 3)));
-  };
+  auto sample = [&](int byte_off) { return pcm_pick<FMT>(sw, byte_off); };
   if (g.planes == 1) {
     float* __restrict__ dst = g.out + clip * g.out_stride + f0;
     for (int f = threadIdx.x; f < tf; f += kPcmThreads) {
-      const int o = skew + f * bpf;
-      float acc = m.w[0] * sample(o);
-      for (int c = 1; c < g.channels; ++c) acc = fmaf(m.w[c], sample(o + c * SB), acc);
-      dst[f] = acc;
+      dst[f] = pcm_mono<FMT>(sw, skew + f * bpf, g.channels, m);
     }
   } else {
     float* __restrict__ dst = g.out + clip * g.planes * g.out_stride + f0;

@@ -121,6 +121,9 @@ struct PcmGeom;
 struct PcmMix;
 int pcm_tile_frames(int bytes_per_frame);
 int launch_pcm_ingest(int format, const PcmGeom& g, long long n_clips, const PcmMix& m, cudaStream_t st);
+// tu_resample.cu: PCM ingestion + polyphase resampling (kernel_resample.cuh); tile_out and tiles are set by the launcher
+struct RsGeom;
+int launch_pcm_resample(int format, RsGeom g, long long n_clips, const PcmMix& m, cudaStream_t st);
 
 #ifdef SG_DEBUG
 int dbg_attach_w32x2p(const DbgState& st);

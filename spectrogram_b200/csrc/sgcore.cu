@@ -21,8 +21,10 @@
 #include "kernel_misc.cuh"
 #include "kernel_w32x2s.cuh"
 #include "kernel_pcm.cuh"
+#include "kernel_resample.cuh"
 #include "plans.cuh"
 using sg::PcmMix; using sg::PcmGeom; using sg::kPcmMaxChannels; using sg::pcm_tile_frames; using sg::launch_pcm_ingest;
+using sg::RsGeom; using sg::launch_pcm_resample;
 
 namespace {
 
@@ -320,6 +322,12 @@ struct PinBuf {
   void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
 };
 
+// Polyphase filter of one reduced ratio up/down (sg_pcm.inl designs it): [up][J] float32 taps, phase-major
+struct RsTable {
+  int up = 1, down = 1, half = 0, J = 0;
+  DevBuf taps;
+};
+
 bool is_pinned(const void* p) {
   cudaPointerAttributes a;
   if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -343,6 +351,7 @@ struct sg_engine {
   DevBuf xs_carry, xs_flags, xs_state;         // fused-smoothing kernel: per-segment carry vectors and their ready flags
   unsigned xs_epoch = 0;
   DevBuf d_raw[2];                   // interleaved PCM bytes in flight (sg_stft_pcm)
+  std::map<std::pair<int, int>, RsTable> rs_tables;   // resampling filters by (up, down)
   PinBuf pin_in[2], pin_out[2];
   int64_t launches = 0;
   int kernel_variant = 0;            // 0 auto, 1 force generic smem kernel
@@ -847,6 +856,7 @@ int sg_engine_destroy(sg_engine* e) {
   cudaFree(e->lut_ref);
   e->lut_user.release(); e->scratch_mag.release(); e->scratch_state.release(); e->scratch_carry.release(); e->xs_carry.release(); e->xs_flags.release(); e->xs_state.release(); e->d_in.release(); e->d_out.release();
   e->d_raw[0].release(); e->d_raw[1].release();
+  for (auto& kv : e->rs_tables) kv.second.taps.release();
   for (int i = 0; i < 2; ++i) { e->pin_in[i].release(); e->pin_out[i].release(); }
   if (e->stream) cudaStreamDestroy(e->stream);
   if (e->s_h2d) cudaStreamDestroy(e->s_h2d);
@@ -931,10 +941,47 @@ int sg_stft_batch_device(sg_engine* e, const float* pcm_dev, int64_t n_clips, in
 namespace {
 // Interleaved PCM in front of the pipeline (sg_stft_pcm): the raw bytes are what is copied to the device, an
 // ingest kernel turns each chunk into float32 planes, and every plane is a clip for the frame kernels.
+// With `rs` set the ingest kernel also resamples: clip_len counts output frames, in_frames the source's.
 struct RawPcm {
   int format, channels, planes, bytes_per_frame;
   PcmMix mix;
+  const RsTable* rs = nullptr;
+  long long in_frames = 0;
 };
+
+long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+// source frames [lo, hi) that outputs [k_lo, k_hi) of a clip of `frames` source frames read (nonzero taps only)
+void resample_input_range(const RsTable& t, long long frames, long long k_lo, long long k_hi, long long* lo, long long* hi) {
+  *lo = std::max(0LL, -floor_div(t.half - k_lo * t.down, t.up));   // ceil((k_lo*down - half)/up)
+  *hi = std::min(frames, floor_div((k_hi - 1) * t.down + t.half, t.up) + 1);
+  if (*hi < *lo) *hi = *lo;
+}
+
+// enqueues the fused ingest + resample kernel: outputs [k0, k0 + n_out) of every plane from source frames
+// [in_f0, in_f0 + in_n) of every clip (clip c's first present frame at src + c*clip_bytes)
+int resample_on_device(sg_engine* e, const RsTable& t, const void* src, long long src_bytes, long long clip_bytes, int64_t n_clips,
+                       long long in_f0, long long in_n, const RawPcm& raw, long long k0, long long n_out, float* out,
+                       long long out_stride, cudaStream_t st) {
+  if (n_clips == 0 || n_out == 0) return SG_OK;
+  RsGeom g;
+  g.src = (const unsigned char*)src;
+  g.src_bytes = src_bytes;
+  g.clip_bytes = clip_bytes;
+  g.in_f0 = in_f0;
+  g.in_n = in_n;
+  g.k0 = k0;
+  g.n_out = n_out;
+  g.out = out;
+  g.out_stride = out_stride;
+  g.taps = (const float*)t.taps.p;
+  g.up = t.up; g.down = t.down; g.half = t.half; g.J = t.J;
+  g.channels = raw.channels;
+  g.planes = raw.planes;
+  SG_CUDA((cudaError_t)launch_pcm_resample(raw.format, g, n_clips, raw.mix, st));
+  e->launches++;
+  return SG_OK;
+}
 
 int stft_batch_impl(sg_engine* e, const void* pcm, int64_t n_clips, int64_t clip_len, const sg_stft_config* cfg,
                     void* out, const RawPcm* raw) {
@@ -955,7 +1002,10 @@ int stft_batch_impl(sg_engine* e, const void* pcm, int64_t n_clips, int64_t clip
   const int bins = cfg->n_fft / 2;
   const size_t eb = elem_bytes(cfg->output);
   const int planes = raw ? raw->planes : 1;               // device clips per source clip
-  const size_t unit = raw ? (size_t)raw->bytes_per_frame : sizeof(float);   // source bytes per sample frame
+  const RsTable* rs = raw ? raw->rs : nullptr;
+  // source bytes per sample frame of the clip (with resampling: per output frame, rounded up)
+  const size_t unit = rs ? ((size_t)raw->bytes_per_frame * rs->down + rs->up - 1) / rs->up
+                         : raw ? (size_t)raw->bytes_per_frame : sizeof(float);
   const size_t out_bytes = (size_t)n_clips * planes * frames * bins * eb;
   // device-resident copies of the whole problem (clip_stride padded to 4 floats for 16-byte rows)
   const long long stride = (clip_len + 3) & ~3LL;
@@ -976,7 +1026,7 @@ int stft_batch_impl(sg_engine* e, const void* pcm, int64_t n_clips, int64_t clip
   const size_t kChunk = kChunkEnv ? kChunkEnv : (size_t)32 << 20;
   struct Chunk { long long c0, nc, t0, nt; };
   std::vector<Chunk> chunks;
-  const size_t clip_bytes = (size_t)clip_len * unit;
+  const size_t clip_bytes = rs ? (size_t)raw->in_frames * raw->bytes_per_frame : (size_t)clip_len * unit;
   const size_t clip_out_bytes = (size_t)planes * frames * bins * eb;
   if (std::max(clip_bytes, clip_out_bytes) <= kChunk) {
     const long long per = std::max<long long>(1, (long long)(kChunk / std::max<size_t>(std::max(clip_bytes, clip_out_bytes), 1)));
@@ -1019,9 +1069,14 @@ int stft_batch_impl(sg_engine* e, const void* pcm, int64_t n_clips, int64_t clip
         s_hi = std::min<long long>(clip_len, std::max<long long>(s_lo, start_base + (ch.t0 + ch.nt - 1) * cfg->hop + cfg->n_fft));
         uploaded_to = s_hi;
       }
-      const size_t row = (size_t)(s_hi - s_lo) * unit;
+      long long in_lo = s_lo, in_hi = s_hi;  // source frames uploaded (differ from s_lo, s_hi when resampling)
+      if (rs) {
+        if (ch.nt == frames) { in_lo = 0; in_hi = raw->in_frames; }
+        else resample_input_range(*rs, raw->in_frames, s_lo, s_hi, &in_lo, &in_hi);
+      }
+      const size_t row = rs ? (size_t)(in_hi - in_lo) * raw->bytes_per_frame : (size_t)(s_hi - s_lo) * unit;
       if (row > 0) {
-        const char* src = (const char*)pcm + (size_t)ch.c0 * clip_bytes + (size_t)s_lo * unit;
+        const char* src = (const char*)pcm + (size_t)ch.c0 * clip_bytes + (size_t)in_lo * (rs ? raw->bytes_per_frame : unit);
         char* dst = (char*)(d_in + ch.c0 * stride + s_lo);   // float32 source: straight into the clip rows
         size_t dpitch = (size_t)stride * sizeof(float);
         if (raw) {                                            // raw PCM: dense rows in this slot's byte buffer
@@ -1048,7 +1103,10 @@ int stft_batch_impl(sg_engine* e, const void* pcm, int64_t n_clips, int64_t clip
       SG_CUDA(cudaEventRecord(ev_in[i & 3], e->s_h2d));
       // ---- kernels
       SG_CUDA(cudaStreamWaitEvent(e->stream, ev_in[i & 3], 0));
-      if (raw && row > 0) {
+      if (rs && s_hi > s_lo) {
+        SG_TRY(resample_on_device(e, *rs, e->d_raw[slot].p, (long long)(row * ch.nc), (long long)row, ch.nc, in_lo, in_hi - in_lo,
+                                  *raw, s_lo, s_hi - s_lo, d_in + ch.c0 * planes * stride + s_lo, stride, e->stream));
+      } else if (raw && row > 0) {
         PcmGeom pg;
         pg.src = (const unsigned char*)e->d_raw[slot].p;
         pg.src_bytes = (long long)(row * ch.nc);

@@ -220,7 +220,8 @@ class AudioBuffer {
 }
 
 // context.decodeAudioData(arrayBuffer, onBuffer, onError) (util/util.js:9-17) for RIFF/WAVE files holding PCM.
-// Keeps the callback form the reference uses and also returns a Promise, like the browser's.
+// Keeps the callback form the reference uses and also returns a Promise, like the browser's.  options.sampleRate is
+// the context's rate (new AudioContext({sampleRate})): a file at another rate is resampled to it on the GPU.
 function decodeAudioData(arrayBuffer, onBuffer, onError, options) {
   const o = options || {};
   return new Promise((resolve, reject) => {
@@ -229,9 +230,17 @@ function decodeAudioData(arrayBuffer, onBuffer, onError, options) {
       const info = guard(native.wavParse)(file);
       const bytes = info.length * info.channels * { u8: 1, s16: 2, s24: 3, s32: 4, f32: 4 }[info.format];
       const samples = file.subarray(info.dataOffset, info.dataOffset + bytes);
-      const planes = new Float32Array(info.channels * info.length);
-      guard(native.pcmDecode)(engineFor(o.device || 0), samples, info, 1, 0, planes);
-      const buffer = new AudioBuffer(planes, info.channels, info.length, info.sampleRate);
+      let buffer;
+      if (o.sampleRate && o.sampleRate !== info.sampleRate) {
+        const length = guard(native.resampleNumFrames)(info.length, info.sampleRate, o.sampleRate);
+        const planes = new Float32Array(info.channels * length);
+        guard(native.pcmDecodeResampled)(engineFor(o.device || 0), samples, info, 1, 0, o.sampleRate, planes);
+        buffer = new AudioBuffer(planes, info.channels, length, o.sampleRate);
+      } else {
+        const planes = new Float32Array(info.channels * info.length);
+        guard(native.pcmDecode)(engineFor(o.device || 0), samples, info, 1, 0, planes);
+        buffer = new AudioBuffer(planes, info.channels, info.length, info.sampleRate);
+      }
       if (onBuffer) onBuffer(buffer);
       resolve(buffer);
     } catch (err) {
@@ -244,10 +253,13 @@ function decodeAudioData(arrayBuffer, onBuffer, onError, options) {
 // The frame path fed with interleaved PCM (Uint8Array view of the samples): ingest and, by default, the
 // AnalyserNode's mono down-mix run on the GPU in front of the batched path.
 // pcm = {format: 'u8'|'s16'|'s24'|'s32'|'f32', channels, sampleRate}; returns {frames, bins, planes, data}.
+// options.sampleRate (the context's rate) resamples from pcm.sampleRate before framing when the two differ.
 function spectrogramPcm(samples, pcm, options) {
   const o = Object.assign({ fftSize: 2048, hop: 512, output: 'u8', mix: true, clips: 1 }, options || {});
   const bytesPerFrame = (pcm.channels || 1) * { u8: 1, s16: 2, s24: 3, s32: 4, f32: 4 }[pcm.format];
-  const length = Math.floor(samples.length / (bytesPerFrame * o.clips));
+  const resample = !!o.sampleRate && o.sampleRate !== pcm.sampleRate;
+  let length = Math.floor(samples.length / (bytesPerFrame * o.clips));
+  if (resample) length = guard(native.resampleNumFrames)(length, pcm.sampleRate || 0, o.sampleRate);
   const frames = guard(native.numFrames)(o, length);
   const bins = o.fftSize / 2;
   const planes = o.mix ? 1 : (pcm.channels || 1);
@@ -255,7 +267,8 @@ function spectrogramPcm(samples, pcm, options) {
   const Ctor = OUT_CTOR[o.output];
   if (!Ctor) throw new TypeError('unknown output ' + o.output);
   const data = new Ctor(n);
-  guard(native.stftPcm)(engineFor(o.device || 0), samples, pcm, o.clips, o.mix ? 1 : 0, o, data);
+  if (resample) guard(native.stftPcmResampled)(engineFor(o.device || 0), samples, pcm, o.clips, o.mix ? 1 : 0, o.sampleRate, o, data);
+  else guard(native.stftPcm)(engineFor(o.device || 0), samples, pcm, o.clips, o.mix ? 1 : 0, o, data);
   return { frames, bins, planes, data };
 }
 

@@ -619,6 +619,81 @@ static napi_value js_stft_pcm(napi_env env, napi_callback_info info) {
   return undefined_of(env);
 }
 
+/* resampleNumFrames(frames, inRate, outRate) -> the length after resampling: ceil(frames*up/down); host only */
+static napi_value js_resample_num_frames(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS], r;
+  int64_t frames, n;
+  int32_t in_rate, out_rate;
+  if (get_args(env, info, argv) < 3 || napi_get_value_int64(env, argv[0], &frames) != napi_ok ||
+      napi_get_value_int32(env, argv[1], &in_rate) != napi_ok || napi_get_value_int32(env, argv[2], &out_rate) != napi_ok)
+    return type_error(env, "resampleNumFrames(frames, inRate, outRate)");
+  n = sg_resample_num_frames(frames, in_rate, out_rate);
+  if (n < 0) return throw_status(env, (int)n);
+  napi_create_double(env, (double)n, &r);
+  return r;
+}
+
+/* pcmDecodeResampled(engine, samples, pcm, nClips, mix, outRate, out: Float32Array): pcmDecode, resampled from
+ * pcm.sampleRate to outRate (decodeAudioData in a context running at outRate); out [clip][plane][resampled frame] */
+static napi_value js_pcm_decode_resampled(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  void *e, *bytes, *out;
+  size_t n, n_out;
+  int32_t n_clips, out_rate;
+  int32_t mix = 0;
+  sg_pcm_info pi;
+  int64_t length;
+  int rc, planes;
+  if (get_args(env, info, argv) < 7 || !get_external(env, argv[0], &e))
+    return type_error(env, "pcmDecodeResampled(engine, samples, pcm, nClips, mix, outRate, out)");
+  if (!get_typed(env, argv[1], napi_uint8_array, &bytes, &n)) return type_error(env, "samples must be a Uint8Array");
+  if (napi_get_value_int32(env, argv[3], &n_clips) != napi_ok) return type_error(env, "nClips must be an integer");
+  if (!parse_pcm(env, argv[2], n, n_clips, &pi)) return undefined_of(env);
+  if (napi_get_value_int32(env, argv[4], &mix) != napi_ok) return type_error(env, "mix must be 0 or 1");
+  if (napi_get_value_int32(env, argv[5], &out_rate) != napi_ok) return type_error(env, "outRate must be an integer");
+  length = sg_resample_num_frames(pi.frames, pi.sample_rate, out_rate);
+  if (length < 0) return throw_status(env, (int)length);
+  if (!get_typed(env, argv[6], napi_float32_array, &out, &n_out)) return type_error(env, "out must be a Float32Array");
+  planes = mix ? 1 : pi.channels;
+  if (n_out < (size_t)n_clips * (size_t)planes * (size_t)length) return type_error(env, "out is smaller than clips x planes x resampled frames");
+  rc = sg_pcm_ingest_resampled((sg_engine*)e, bytes, n_clips, &pi, mix ? SG_PCM_MONO_MIX : SG_PCM_PLANAR, out_rate, (float*)out);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
+/* stftPcmResampled(engine, samples, pcm, nClips, mix, outRate, options, out): stftPcm with the planes resampled
+ * from pcm.sampleRate to outRate before framing */
+static napi_value js_stft_pcm_resampled(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  void *e, *bytes, *out;
+  size_t n, n_out;
+  int32_t n_clips, out_rate;
+  int32_t mix = 1;
+  sg_pcm_info pi;
+  sg_stft_config cfg;
+  int64_t length, frames;
+  int rc, planes;
+  if (get_args(env, info, argv) < 8 || !get_external(env, argv[0], &e))
+    return type_error(env, "stftPcmResampled(engine, samples, pcm, nClips, mix, outRate, options, out)");
+  if (!get_typed(env, argv[1], napi_uint8_array, &bytes, &n)) return type_error(env, "samples must be a Uint8Array");
+  if (napi_get_value_int32(env, argv[3], &n_clips) != napi_ok) return type_error(env, "nClips must be an integer");
+  if (!parse_pcm(env, argv[2], n, n_clips, &pi)) return undefined_of(env);
+  if (napi_get_value_int32(env, argv[4], &mix) != napi_ok) return type_error(env, "mix must be 0 or 1");
+  if (napi_get_value_int32(env, argv[5], &out_rate) != napi_ok) return type_error(env, "outRate must be an integer");
+  if (!parse_config(env, argv[6], &cfg)) return undefined_of(env);
+  length = sg_resample_num_frames(pi.frames, pi.sample_rate, out_rate);
+  if (length < 0) return throw_status(env, (int)length);
+  frames = sg_stft_num_frames(&cfg, length);
+  if (frames < 0) return throw_status(env, SG_ERR_INDEX_SIZE);
+  planes = mix ? 1 : pi.channels;
+  if (!get_typed(env, argv[7], sg_stft_elem_bytes(&cfg) == 1 ? napi_uint8_array : (cfg.output == SG_OUT_RGBA8 ? napi_uint32_array : napi_float32_array), &out, &n_out))
+    return type_error(env, "out has the wrong element type for options.output");
+  if (n_out < (size_t)n_clips * (size_t)planes * (size_t)frames * (size_t)(cfg.n_fft / 2)) return type_error(env, "out is smaller than clips x planes x frames x bins");
+  rc = sg_stft_pcm_resampled((sg_engine*)e, bytes, n_clips, &pi, mix ? SG_PCM_MONO_MIX : SG_PCM_PLANAR, out_rate, &cfg, out);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
 /* ---------------------------------------------------------------- module init */
 static void export_fn(napi_env env, napi_value exports, const char* name, napi_callback cb) {
   napi_value fn;
@@ -656,6 +731,9 @@ napi_value napi_register_module_v1(napi_env env, napi_value exports) {
   export_fn(env, exports, "wavParse", js_wav_parse);
   export_fn(env, exports, "pcmDecode", js_pcm_decode);
   export_fn(env, exports, "stftPcm", js_stft_pcm);
+  export_fn(env, exports, "resampleNumFrames", js_resample_num_frames);
+  export_fn(env, exports, "pcmDecodeResampled", js_pcm_decode_resampled);
+  export_fn(env, exports, "stftPcmResampled", js_stft_pcm_resampled);
   return exports;
 }
 
