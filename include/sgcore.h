@@ -197,15 +197,37 @@ int sg_analyser_get_float_time_domain_data(sg_analyser* a, float* dst, int64_t l
 int sg_stream_create(sg_engine* e, int n_channels, const sg_stft_config* cfg, int max_chunk,
                      sg_stream** out);
 int sg_stream_destroy(sg_stream* s);
-int sg_stream_reset(sg_stream* s); /* zero history and smoothing state */
+int sg_stream_reset(sg_stream* s); /* zero history and smoothing state, and clear an attached sonogram history */
 /* chunk: host [n_channels][chunk_len] float32, chunk_len a multiple of hop.
- * out: host [n_channels][chunk_len/hop][bins] elements of cfg.output.
+ * out: host [n_channels][chunk_len/hop][bins] elements of cfg.output.  It may be NULL when a
+ * sonogram history is attached (sg_stream_set_history): the rows then only land in the history.
  * out_rgba (may be NULL): additionally host [n_channels][chunk_len/hop][bins] RGBA8 through the
- * colour LUT (only when cfg.output == SG_OUT_U8).  Synchronous: returns when both are filled. */
+ * colour LUT (only when cfg.output == SG_OUT_U8, and only with out).  Synchronous: returns when
+ * both are filled and the history holds the new rows. */
 int sg_stream_push(sg_stream* s, const float* chunk, int chunk_len, void* out, uint32_t* out_rgba);
 int64_t sg_stream_frames_emitted(const sg_stream* s); /* per channel */
 /* geometry of a stream object (any pointer may be NULL): what a binding needs to check the caller's array lengths */
 int sg_stream_info(const sg_stream* s, int* channels, int* hop, int* bins, int* output, int* max_chunk);
+
+/* Sonogram history of a stream: per channel, what an sg_ring(bins, rows) holds when it is fed
+ * every push's byte rows, kept on the device and filled there (device-to-device) by each push.
+ * Texture [n_channels][rows][bins] u8; the channels share one yoffset.  Needs cfg.output ==
+ * SG_OUT_U8 (else SG_ERR_INVALID_ARG).  rows in [2, 65536], or 0 to detach (else
+ * SG_ERR_INVALID_ARG).  Attaching, even with the current row count, starts it empty: texture
+ * zero, yoffset 0 (initByteBuffer, visualizer.js:317-329). */
+int sg_stream_set_history(sg_stream* s, int rows);
+/* rows = 0 when no history is attached; either pointer may be NULL */
+int sg_stream_history_info(const sg_stream* s, int* rows, int* yoffset);
+/* channels [first, first+count) of the texture, host [count][rows][bins], texture row order
+ * (each channel equals sg_ring_read of its ring) */
+int sg_stream_history_read(sg_stream* s, int first, int count, uint8_t* dst);
+/* sg_ring_view of channels [first, first+count) in one launch: host [count][height][width] RGBA8,
+ * each image bit-identical to sg_ring_view of that channel's ring.  Page-locked rgba_out is
+ * written by DMA directly.  Errors: SG_ERR_INVALID_ARG for a NULL pointer, width or height < 1,
+ * width * height > 2^28, count * width * height > 2^30, or a channel range outside
+ * [0, n_channels) or empty; then SG_ERR_STATE when no history is attached.  The same channel
+ * range and state rules apply to sg_stream_history_read. */
+int sg_stream_view(sg_stream* s, int first, int count, int width, int height, uint32_t* rgba_out);
 
 /* ------------------------------------------------------------------ PCM ingestion ---------- */
 /* The step in front of the path: the reference hands an encoded file to the browser,

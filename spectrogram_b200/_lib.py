@@ -38,6 +38,13 @@ class EngineError(RuntimeError):
     """CUDA failure, out of memory, or no device (the engine has no CPU path)."""
 
 
+class InvalidStateError(RuntimeError):
+    """Web platform ``InvalidStateError`` DOMException: the call is not valid in the object's current state
+    (``SG_ERR_STATE``, e.g. a sonogram view of a stream bank without a history)."""
+
+    name = "InvalidStateError"
+
+
 class StftConfig(C.Structure):
     """``sg_stft_config``."""
 
@@ -102,6 +109,10 @@ SIGNATURES = {
     "sg_stream_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "sg_stream_frames_emitted": (C.c_int64, [C.c_void_p]),
     "sg_stream_info": (C.c_int, [C.c_void_p] + [C.POINTER(C.c_int)] * 5),
+    "sg_stream_set_history": (C.c_int, [C.c_void_p, C.c_int]),
+    "sg_stream_history_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "sg_stream_history_read": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "sg_stream_view": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "sg_pcm_sample_bytes": (C.c_int, [C.c_int]),
     "sg_pcm_num_planes": (C.c_int, [C.POINTER(PcmInfo), C.c_int]),
     "sg_wav_parse": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(PcmInfo)]),
@@ -162,4 +173,6 @@ def check(rc: int) -> None:
         raise TypeError(msg)
     if rc == SG_ERR_OOM:
         raise MemoryError(msg)
+    if rc == SG_ERR_STATE:
+        raise InvalidStateError(msg)
     raise EngineError(f"sg_status {rc}: {msg}")

@@ -356,9 +356,14 @@ class PinnedArray:
 
 
 class StreamBank:
-    """``sg_stream``: n_channels analysers advanced in lock step (BASELINE config 5)."""
+    """``sg_stream``: n_channels analysers advanced in lock step (BASELINE config 5).
 
-    def __init__(self, n_channels: int, opts: Options, max_chunk: int | None = None, engine: Engine | None = None):
+    ``history_rows``: keep a sonogram history per channel on the device (``sg_stream_set_history``) -- what a
+    ``SonogramRing(bins, history_rows)`` fed every push's byte rows would hold -- so ``view()`` renders every channel's
+    picture in one launch without the rows crossing PCIe twice.  Needs ``output="u8"``."""
+
+    def __init__(self, n_channels: int, opts: Options, max_chunk: int | None = None, engine: Engine | None = None,
+                 history_rows: int | None = None):
         self.engine = engine or default_engine(0)
         self._lib = L.load()
         self.opts = opts
@@ -369,6 +374,8 @@ class StreamBank:
         h = C.c_void_p()
         L.check(self._lib.sg_stream_create(self.engine.handle, self.n_channels, C.byref(cfg), self.max_chunk, C.byref(h)))
         self._h = h
+        if history_rows is not None:
+            self.set_history(history_rows)
 
     def push(self, chunk, out=None, out_rgba=None, want_rgba: bool = False):
         x = np.ascontiguousarray(chunk, dtype=np.float32)
@@ -385,8 +392,58 @@ class StreamBank:
                                          out_rgba.ctypes.data if out_rgba is not None else None))
         return (out, out_rgba) if out_rgba is not None else out
 
+    def advance(self, chunk) -> None:
+        """``push`` whose byte rows only go to the sonogram history: nothing is copied back to the host."""
+        x = np.ascontiguousarray(chunk, dtype=np.float32)
+        if x.ndim != 2 or x.shape[0] != self.n_channels:
+            raise TypeError("chunk must be [n_channels, chunk_len]")
+        L.check(self._lib.sg_stream_push(self._h, x.ctypes.data, x.shape[1], None, None))
+
     def reset(self):
         L.check(self._lib.sg_stream_reset(self._h))
+
+    # -- sonogram history ----------------------------------------------------------------------
+    def set_history(self, rows: int) -> None:
+        """Attach an empty history of ``rows`` rows per channel ([2, 65536]); 0 detaches it."""
+        L.check(self._lib.sg_stream_set_history(self._h, int(rows)))
+
+    def _history_info(self):
+        rows, y = C.c_int(), C.c_int()
+        L.check(self._lib.sg_stream_history_info(self._h, C.byref(rows), C.byref(y)))
+        return rows.value, y.value
+
+    @property
+    def history_rows(self) -> int:
+        return self._history_info()[0]
+
+    @property
+    def history_yoffset(self) -> int:
+        return self._history_info()[1]
+
+    def _range(self, first, count):
+        first = int(first)
+        return first, (self.n_channels - first if count is None else int(count))
+
+    def history(self, first: int = 0, count: int | None = None) -> np.ndarray:
+        """Textures of channels [first, first+count): uint8 [count, rows, bins] in texture row order."""
+        first, count = self._range(first, count)
+        rows = self.history_rows
+        out = np.empty((max(count, 0), rows, self._cfg.n_fft // 2), dtype=np.uint8)
+        L.check(self._lib.sg_stream_history_read(self._h, first, count, out.ctypes.data))
+        return out
+
+    def view(self, width: int, height: int, first: int = 0, count: int | None = None,
+             out: np.ndarray | None = None) -> np.ndarray:
+        """Sonogram pictures of channels [first, first+count), one launch: RGBA8 [count, height, width, 4], each equal
+        to ``SonogramRing.view`` of that channel's ring."""
+        first, count = self._range(first, count)
+        shape = (max(count, 0), max(int(height), 0), max(int(width), 0), 4)
+        if out is None:
+            out = np.empty(shape, dtype=np.uint8)
+        elif out.dtype != np.uint8 or out.shape != shape or not out.flags.c_contiguous:
+            raise TypeError(f"out must be C-contiguous uint8 {shape}")
+        L.check(self._lib.sg_stream_view(self._h, first, count, int(width), int(height), out.ctypes.data))
+        return out
 
     @property
     def frames_emitted(self) -> int:

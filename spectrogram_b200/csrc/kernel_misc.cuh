@@ -195,12 +195,10 @@ __global__ void time_domain_byte_kernel(const float* __restrict__ x, uint8_t* __
 //   rgb = HSV(360 - 360 a, 1, 1)          sonogram-vertex.shader:19-58 (evaluated per pixel here, per vertex there)
 //   fade = sqrt(cos((1-v) pi/2))          fragment:24
 //   out = clamp(0.08 + a*fade*rgb), alpha 1, 8-bit round-to-nearest            fragment:26, visualizer.js:69
-__global__ void __launch_bounds__(256)
-sonogram_view_kernel(const uint8_t* __restrict__ ring, int bins, int rows, int yoffset, int width, int height,
-                     float background, uint32_t* __restrict__ out) {
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (long long)width * height) return;
-  const int py = (int)(idx / width), px = (int)(idx - (long long)py * width);
+// One pixel of that picture, from a [rows][bins] texture.  Shared by the single view and the batched one below so the
+// two stay bit-identical: every term is evaluated in the same order on both paths.
+__device__ __forceinline__ uint32_t sonogram_pixel(const uint8_t* __restrict__ ring, int bins, int rows, int yoffset,
+                                                   int px, int py, int width, int height, float background) {
   const float u = (px + 0.5f) / width, v = (py + 0.5f) / height;
   const float sc = exp2f(8.f * (u - 1.f));                       // 256^(u-1)
   float tc = v + (float)yoffset / (float)(rows - 1);
@@ -226,7 +224,50 @@ sonogram_view_kernel(const uint8_t* __restrict__ ring, int bins, int rows, int y
   else if (hd < 6.f) { r = 1.f; b = xx; }
   const float k = a * sqrtf(fmaxf(cospif((1.f - v) * 0.5f), 0.f));
   auto q = [&](float c) { return (uint32_t)floorf(fminf(fmaxf(fmaf(k, c, background), 0.f), 1.f) * 255.f + 0.5f); };
-  out[idx] = q(r) | (q(g) << 8) | (q(b) << 16) | 0xFF000000u;
+  return q(r) | (q(g) << 8) | (q(b) << 16) | 0xFF000000u;
+}
+
+__global__ void __launch_bounds__(256)
+sonogram_view_kernel(const uint8_t* __restrict__ ring, int bins, int rows, int yoffset, int width, int height,
+                     float background, uint32_t* __restrict__ out) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)width * height) return;
+  const int py = (int)(idx / width), px = (int)(idx - (long long)py * width);
+  out[idx] = sonogram_pixel(ring, bins, rows, yoffset, px, py, width, height, background);
+}
+
+// The same picture for `count` textures that share rows and yoffset (a streaming bank's channels), in one launch.
+// tex: [count][rows][bins] u8; out: [count][height][width] RGBA8, from cudaMalloc (16-byte aligned).
+// A thread owns four neighbouring pixels of one image row and walks channels [blockIdx.y*per, +per): everything in
+// sonogram_pixel but the four texel loads and what follows them is the same for every channel, so the compiler hoists
+// it out of the channel loop, and each pixel's arithmetic is still exactly sonogram_view_kernel's.
+// Stores are one 16-byte store per thread and channel when width % 4 == 0 (each image row then starts 16-byte aligned).
+__global__ void __launch_bounds__(256)
+sonogram_views_kernel(const uint8_t* __restrict__ tex, int count, int per, int bins, int rows, int yoffset, int width,
+                      int height, float background, uint32_t* __restrict__ out) {
+  const int qw = (width + 3) >> 2;
+  const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= (long long)qw * height) return;
+  const int py = (int)(q / qw), px = (int)(q - (long long)py * qw) * 4;
+  const int c0 = blockIdx.y * per, c1 = min(count, c0 + per);
+  const long long plane = (long long)rows * bins, img = (long long)width * height, o0 = (long long)py * width + px;
+  if ((width & 3) == 0) {
+    for (int c = c0; c < c1; ++c) {
+      const uint8_t* t = tex + c * plane;
+      const uint4 v = make_uint4(sonogram_pixel(t, bins, rows, yoffset, px, py, width, height, background),
+                                 sonogram_pixel(t, bins, rows, yoffset, px + 1, py, width, height, background),
+                                 sonogram_pixel(t, bins, rows, yoffset, px + 2, py, width, height, background),
+                                 sonogram_pixel(t, bins, rows, yoffset, px + 3, py, width, height, background));
+      *reinterpret_cast<uint4*>(out + c * img + o0) = v;
+    }
+  } else {
+    const int n = min(4, width - px);
+    for (int c = c0; c < c1; ++c) {
+      const uint8_t* t = tex + c * plane;
+      for (int i = 0; i < n; ++i)
+        out[c * img + o0 + i] = sonogram_pixel(t, bins, rows, yoffset, px + i, py, width, height, background);
+    }
+  }
 }
 
 }  // namespace sg

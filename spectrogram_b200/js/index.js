@@ -150,6 +150,8 @@ function spectrogram(pcm, opts) {
   return { frames, bins, data };
 }
 
+// opts.historyRows keeps a sonogram history per channel on the device: what a SonogramRing(bins, historyRows) fed
+// every push's byte rows would hold.  view() then draws every channel's picture in one launch (output 'u8' only).
 class StreamBank {
   constructor(nChannels, opts, maxChunk) {
     this.opts = Object.assign({ fftSize: 1024, hop: 128, output: 'u8' }, opts || {});
@@ -157,11 +159,44 @@ class StreamBank {
     this.maxChunk = maxChunk || this.opts.hop;
     this._h = guard(native.streamCreate)(engineFor(this.opts.device || 0), nChannels, this.opts, this.maxChunk);
     own(this, native.streamDestroy, this._h);
+    if (this.opts.historyRows) this.setHistory(this.opts.historyRows);
   }
-  // chunk: Float32Array [channel][chunkLen]; out: typed array [channel][chunkLen/hop][bins]
+  // chunk: Float32Array [channel][chunkLen]; out: typed array [channel][chunkLen/hop][bins], or undefined when a
+  // history is attached and only the pictures are wanted (no rows come back to the host)
   push(chunk, out, outRgba) {
     const chunkLen = wholeNumber(chunk.length / this.nChannels, 'chunk.length / nChannels');
     guard(native.streamPush)(this._h, chunk, chunkLen, out, outRgba);
+  }
+  // attach an empty history of `rows` rows per channel (texture zero, yoffset 0); 0 detaches it
+  setHistory(rows) {
+    guard(native.streamSetHistory)(this._h, rows);
+  }
+  get historyRows() {
+    return native.streamHistoryInfo(this._h).rows;
+  }
+  get historyYoffset() {
+    return native.streamHistoryInfo(this._h).yoffset;
+  }
+  _range(o) {
+    const first = o.first || 0;
+    return [first, o.count === undefined ? this.nChannels - first : o.count];
+  }
+  // textures of channels [first, first+count): Uint8Array [count][rows][bins], texture row order
+  history(options) {
+    const o = options || {};
+    const [first, count] = this._range(o);
+    const out = o.out || new Uint8Array(Math.max(count * this.historyRows * (this.opts.fftSize / 2), 0) || 0);
+    guard(native.streamHistoryRead)(this._h, first, count, out);
+    return out;
+  }
+  // RGBA8 pictures of channels [first, first+count) in one launch: Uint32Array [count][height][width], each what
+  // SonogramRing.view draws for that channel
+  view(width, height, options) {
+    const o = options || {};
+    const [first, count] = this._range(o);
+    const out = o.out || new Uint32Array(Math.max(count * width * height, 0) || 0);   // bad sizes are the native's to report
+    guard(native.streamView)(this._h, first, count, width, height, out);
+    return out;
   }
   close() {
     if (this._h) { disown(this); native.streamDestroy(this._h); }

@@ -37,6 +37,7 @@ static napi_value throw_status(napi_env env, int rc) {
   else if (rc == SG_ERR_INVALID_ARG) napi_throw_type_error(env, "ERR_INVALID_ARG_TYPE", msg);
   else if (rc == SG_ERR_NO_DEVICE) napi_throw_error(env, "ERR_NO_CUDA_DEVICE", msg);
   else if (rc == SG_ERR_OOM) napi_throw_error(env, "ERR_OUT_OF_MEMORY", msg);
+  else if (rc == SG_ERR_STATE) napi_throw_error(env, "InvalidStateError", msg);
   else napi_throw_error(env, "ERR_CUDA", msg);
   return undefined_of(env);
 }
@@ -406,20 +407,22 @@ static napi_value js_stream_create(napi_env env, napi_callback_info info) {
   return r;
 }
 
-/* streamPush(stream, chunk: Float32Array, chunkLen, out, outRgba | undefined) */
+/* streamPush(stream, chunk: Float32Array, chunkLen, out | undefined, outRgba | undefined); out may be undefined only
+ * when a sonogram history is attached (the rows then only land in the history) */
 static napi_value js_stream_push(napi_env env, napi_callback_info info) {
   napi_value argv[MAX_ARGS];
-  void *s, *chunk, *out, *rgba = NULL;
-  size_t chunk_n, out_n, rgba_n;
+  void *s, *chunk, *out = NULL, *rgba = NULL;
+  size_t chunk_n, out_n = 0, rgba_n;
   int32_t chunk_len;
   bool is = false;
-  int rc;
+  int rc, have_out;
   size_t argc = get_args(env, info, argv);
   if (argc < 4 || !get_external(env, argv[0], &s)) return type_error(env, "streamPush(stream, chunk, chunkLen, out[, outRgba])");
   if (!get_typed(env, argv[1], napi_float32_array, &chunk, &chunk_n)) return type_error(env, "chunk must be a Float32Array");
   if (napi_get_value_int32(env, argv[2], &chunk_len) != napi_ok) return type_error(env, "chunkLen must be an integer");
-  if (napi_is_typedarray(env, argv[3], &is) != napi_ok || !is ||
-      napi_get_typedarray_info(env, argv[3], NULL, &out_n, &out, NULL, NULL) != napi_ok)
+  have_out = !is_undefined(env, argv[3]);
+  if (have_out && (napi_is_typedarray(env, argv[3], &is) != napi_ok || !is ||
+                   napi_get_typedarray_info(env, argv[3], NULL, &out_n, &out, NULL, NULL) != napi_ok))
     return type_error(env, "out must be a typed array");
   if (argc >= 5 && !is_undefined(env, argv[4]) && !get_typed(env, argv[4], napi_uint32_array, &rgba, &rgba_n))
     return type_error(env, "outRgba must be a Uint32Array");
@@ -433,13 +436,101 @@ static napi_value js_stream_push(napi_env env, napi_callback_info info) {
     if (chunk_len < 0 || chunk_len > max_chunk || chunk_len % hop) return type_error(env, "chunkLen must be a multiple of hop, at most maxChunk");
     if ((uint64_t)chunk_n < (uint64_t)channels * (uint64_t)chunk_len) return type_error(env, "chunk is shorter than channels * chunkLen");
     need = (uint64_t)channels * (uint64_t)(chunk_len / hop) * (uint64_t)bins;
-    napi_get_typedarray_info(env, argv[3], &got, NULL, NULL, NULL, NULL);
-    if (got != (output == SG_OUT_U8 ? napi_uint8_array : (output == SG_OUT_RGBA8 ? napi_uint32_array : napi_float32_array)))
-      return type_error(env, "out has the wrong typed-array type for this stream's output");
-    if ((uint64_t)out_n < need) return type_error(env, "out is shorter than channels * frames * bins");
-    if (rgba && (uint64_t)rgba_n < need) return type_error(env, "outRgba is shorter than channels * frames * bins");
+    if (have_out) {
+      napi_get_typedarray_info(env, argv[3], &got, NULL, NULL, NULL, NULL);
+      if (got != (output == SG_OUT_U8 ? napi_uint8_array : (output == SG_OUT_RGBA8 ? napi_uint32_array : napi_float32_array)))
+        return type_error(env, "out has the wrong typed-array type for this stream's output");
+      if ((uint64_t)out_n < need) return type_error(env, "out is shorter than channels * frames * bins");
+      if (rgba && (uint64_t)rgba_n < need) return type_error(env, "outRgba is shorter than channels * frames * bins");
+    } else {
+      int rows = 0;
+      if (sg_stream_history_info((sg_stream*)s, &rows, NULL) != SG_OK || !rows)
+        return type_error(env, "out must be a typed array (it may be undefined only when a history is attached)");
+      if (rgba) return type_error(env, "outRgba needs out");
+    }
   }
   rc = sg_stream_push((sg_stream*)s, (const float*)chunk, chunk_len, out, (uint32_t*)rgba);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
+/* streamSetHistory(stream, rows): attach an empty sonogram history of rows rows per channel, or detach it (rows 0) */
+static napi_value js_stream_set_history(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  void* s;
+  int32_t rows;
+  int rc;
+  if (get_args(env, info, argv) < 2 || !get_external(env, argv[0], &s)) return type_error(env, "streamSetHistory(stream, rows)");
+  if (napi_get_value_int32(env, argv[1], &rows) != napi_ok) return type_error(env, "rows must be an integer");
+  rc = sg_stream_set_history((sg_stream*)s, rows);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
+/* streamHistoryInfo(stream) -> {rows, yoffset}; rows is 0 when no history is attached */
+static napi_value js_stream_history_info(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS], o;
+  void* s;
+  int rows = 0, yoffset = 0;
+  if (get_args(env, info, argv) < 1 || !get_external(env, argv[0], &s)) return type_error(env, "stream expected");
+  if (sg_stream_history_info((sg_stream*)s, &rows, &yoffset) != SG_OK) return type_error(env, "stream expected");
+  napi_create_object(env, &o);
+  napi_set_named_property(env, o, "rows", make_int(env, rows));
+  napi_set_named_property(env, o, "yoffset", make_int(env, yoffset));
+  return o;
+}
+
+/* channels [first, first+count) of a stream's history checked against its geometry; 0 and a pending TypeError when the
+ * range is outside the bank.  *rows and *bins get the texture's size (rows 0: no history; the core then reports it). */
+static int history_range(napi_env env, void* s, int32_t first, int32_t count, int* rows, int* bins) {
+  int channels = 0;
+  if (sg_stream_info((sg_stream*)s, &channels, NULL, bins, NULL, NULL) != SG_OK ||
+      sg_stream_history_info((sg_stream*)s, rows, NULL) != SG_OK) {
+    type_error(env, "stream expected");
+    return 0;
+  }
+  if (first < 0 || count < 1 || count > channels - first) {
+    type_error(env, "channel range outside the bank");
+    return 0;
+  }
+  return 1;
+}
+
+/* streamHistoryRead(stream, first, count, out: Uint8Array [count][rows][bins]) */
+static napi_value js_stream_history_read(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  void *s, *out;
+  size_t n;
+  int32_t first, count;
+  int rows = 0, bins = 0, rc;
+  if (get_args(env, info, argv) < 4 || !get_external(env, argv[0], &s)) return type_error(env, "streamHistoryRead(stream, first, count, out)");
+  if (napi_get_value_int32(env, argv[1], &first) != napi_ok || napi_get_value_int32(env, argv[2], &count) != napi_ok)
+    return type_error(env, "first and count must be integers");
+  if (!get_typed(env, argv[3], napi_uint8_array, &out, &n)) return type_error(env, "out must be a Uint8Array");
+  if (!history_range(env, s, first, count, &rows, &bins)) return undefined_of(env);
+  if ((uint64_t)n < (uint64_t)count * (uint64_t)rows * (uint64_t)bins) return type_error(env, "out is shorter than count * rows * bins");
+  rc = sg_stream_history_read((sg_stream*)s, first, count, (uint8_t*)out);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
+/* streamView(stream, first, count, width, height, out: Uint32Array [count][height][width]): every channel's sonogram
+ * picture in one launch */
+static napi_value js_stream_view(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  void *s, *out;
+  size_t n;
+  int32_t first, count, w, h;
+  int rows = 0, bins = 0, rc;
+  if (get_args(env, info, argv) < 6 || !get_external(env, argv[0], &s)) return type_error(env, "streamView(stream, first, count, width, height, out)");
+  if (napi_get_value_int32(env, argv[1], &first) != napi_ok || napi_get_value_int32(env, argv[2], &count) != napi_ok ||
+      napi_get_value_int32(env, argv[3], &w) != napi_ok || napi_get_value_int32(env, argv[4], &h) != napi_ok)
+    return type_error(env, "first, count, width and height must be integers");
+  if (!get_typed(env, argv[5], napi_uint32_array, &out, &n)) return type_error(env, "out must be a Uint32Array");
+  if (w < 1 || h < 1 || (uint64_t)w * (uint64_t)h > (1ull << 28)) return type_error(env, "image size out of range");
+  if (!history_range(env, s, first, count, &rows, &bins)) return undefined_of(env);
+  if ((uint64_t)n < (uint64_t)count * (uint64_t)w * (uint64_t)h) return type_error(env, "out is shorter than count * width * height");
+  rc = sg_stream_view((sg_stream*)s, first, count, w, h, (uint32_t*)out);
   if (rc != SG_OK) return throw_status(env, rc);
   return undefined_of(env);
 }
@@ -723,6 +814,10 @@ napi_value napi_register_module_v1(napi_env env, napi_value exports) {
   export_fn(env, exports, "streamCreate", js_stream_create);
   export_fn(env, exports, "streamPush", js_stream_push);
   export_fn(env, exports, "streamDestroy", js_stream_destroy);
+  export_fn(env, exports, "streamSetHistory", js_stream_set_history);
+  export_fn(env, exports, "streamHistoryInfo", js_stream_history_info);
+  export_fn(env, exports, "streamHistoryRead", js_stream_history_read);
+  export_fn(env, exports, "streamView", js_stream_view);
   export_fn(env, exports, "ringCreate", js_ring_create);
   export_fn(env, exports, "ringAppend", js_ring_append);
   export_fn(env, exports, "ringYoffset", js_ring_yoffset);
