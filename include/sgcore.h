@@ -229,6 +229,76 @@ int sg_stream_history_read(sg_stream* s, int first, int count, uint8_t* dst);
  * range and state rules apply to sg_stream_history_read. */
 int sg_stream_view(sg_stream* s, int first, int count, int width, int height, uint32_t* rgba_out);
 
+/* ------------------------------------------------------------------ biquad filter ---------- */
+/* W3C BiquadFilterNode.  The reference's draw mode (Player.setBandpassFrequency, UI/player.js) puts one in front of
+ * the analyser: type 'bandpass', Q 10, frequency = the band under the pointer, so the sonogram shows only that band.
+ *
+ * Parameters: type (enum below, the spec's order), frequency (Hz, default 350), q (default 1), gain (dB, default 0),
+ * detune (cents, default 0), sample_rate (the context's rate: an integer in [3000, 768000]).  A non-finite parameter, a
+ * bad type or a bad sample_rate is SG_ERR_INVALID_ARG.  f0 = frequency * 2^(detune/1200) clamped to [0, sample_rate/2]
+ * (frequency 0 stays 0 whatever the detune); q and gain take any finite value; gain only matters to lowshelf,
+ * highshelf and peaking.
+ *
+ * Coefficients, in double: w0 = 2 pi f0/Fs, c = cos w0, A = 10^(gain/40);
+ *   aQ = sin w0/(2 q)              (bandpass, notch, allpass, peaking)
+ *   aQdB = sin w0/(2 10^(q/20))    (lowpass, highpass)
+ *   aS = sin w0/sqrt(2)            (the shelves, S = 1)
+ *   type       b0                       b1                  b2                       a0                     a1                   a2
+ *   lowpass    (1-c)/2                  1-c                 (1-c)/2                  1+aQdB                 -2c                  1-aQdB
+ *   highpass   (1+c)/2                  -(1+c)              (1+c)/2                  1+aQdB                 -2c                  1-aQdB
+ *   bandpass   aQ                       0                   -aQ                      1+aQ                   -2c                  1-aQ
+ *   lowshelf   A[(A+1)-(A-1)c+2aS vA]   2A[(A-1)-(A+1)c]    A[(A+1)-(A-1)c-2aS vA]   (A+1)+(A-1)c+2aS vA    -2[(A-1)+(A+1)c]     (A+1)+(A-1)c-2aS vA
+ *   highshelf  A[(A+1)+(A-1)c+2aS vA]   -2A[(A-1)+(A+1)c]   A[(A+1)+(A-1)c-2aS vA]   (A+1)-(A-1)c+2aS vA    2[(A-1)-(A+1)c]      (A+1)-(A-1)c-2aS vA
+ *   peaking    1+aQ A                   -2c                 1-aQ A                   1+aQ/A                 -2c                  1-aQ/A
+ *   notch      1                        -2c                 1                        1+aQ                   -2c                  1-aQ
+ *   allpass    1-aQ                     -2c                 1+aQ                     1+aQ                   -2c                  1-aQ
+ * (vA = sqrt(A)), every coefficient divided by a0.  Where the formulas degenerate the filter is the limit of H(z), a
+ * constant k (b0 = k, b1 = b2 = a1 = a2 = 0):
+ *   f0 = 0:       lowpass, bandpass -> 0;  highpass, lowshelf, peaking, notch, allpass -> 1;  highshelf -> A^2
+ *   f0 = Fs/2:    lowpass, highshelf, peaking, notch, allpass -> 1;  highpass, bandpass -> 0;  lowshelf -> A^2
+ *   q <= 0 with 0 < f0 < Fs/2:  bandpass -> 1;  notch -> 0;  allpass -> -1;  peaking -> A^2
+ *
+ * Filtering is direct form I, y[n] = b0 x[n] + b1 x[n-1] + b2 x[n-2] - a1 y[n-1] - a2 y[n-2], with float64 arithmetic
+ * and float64 state, each output rounded to float32 once.  Per channel the state is {x1, x2, y1, y2} (four doubles;
+ * y unrounded).  The kernel runs each channel along time in parallel, which reorders the double arithmetic: every
+ * output is within 1 float32 ulp of the sequential float64 recurrence rounded to float32, or within 2^-30 max|x| of
+ * the channel, whichever is larger, also when a channel is split over calls with the state carried.  The launches
+ * depend only on (n_channels, len), so equal inputs give bit-identical outputs.  Non-finite samples propagate as
+ * IEEE arithmetic gives. */
+typedef enum sg_biquad_type {
+  SG_BIQUAD_LOWPASS = 0, SG_BIQUAD_HIGHPASS = 1, SG_BIQUAD_BANDPASS = 2, SG_BIQUAD_LOWSHELF = 3,
+  SG_BIQUAD_HIGHSHELF = 4, SG_BIQUAD_PEAKING = 5, SG_BIQUAD_NOTCH = 6, SG_BIQUAD_ALLPASS = 7
+} sg_biquad_type;
+
+typedef struct sg_biquad_params {
+  int32_t type;        /* sg_biquad_type                                                          */
+  double sample_rate;  /* Hz, an integer in [3000, 768000]                                        */
+  double frequency;    /* Hz                                                                      */
+  double q;
+  double gain;         /* dB                                                                      */
+  double detune;       /* cents                                                                   */
+} sg_biquad_params;
+
+/* normalised {b0, b1, b2, a1, a2}; host only, needs no engine */
+int sg_biquad_coefficients(const sg_biquad_params* p, double coef[5]);
+/* in, out: host [n_channels][len] float32 (in == out allowed).  state: host [n_channels][4] doubles {x1, x2, y1, y2},
+ * read as the initial state and written with the final one; NULL = zero start, no write-back.  Synchronous. */
+int sg_biquad_filter(sg_engine* e, const sg_biquad_params* p, const float* in, int64_t n_channels, int64_t len,
+                     double* state, float* out);
+/* Same on device buffers, asynchronous on cuda_stream (NULL = the engine's stream); does not synchronise.  Channel c
+ * reads in_dev + c*in_stride and writes out_dev + c*out_stride (strides >= len).  In place is allowed: in_dev == out_dev
+ * with equal strides; otherwise the two must not overlap.  state_dev: device [n_channels][4] doubles, or NULL.
+ * Channels longer than 4096 samples use three launches and the engine's scratch (ordered like sg_stft_batch_device's). */
+int sg_biquad_filter_device(sg_engine* e, const sg_biquad_params* p, const float* in_dev, int64_t n_channels,
+                            int64_t len, int64_t in_stride, float* out_dev, int64_t out_stride, double* state_dev,
+                            void* cuda_stream);
+/* The bank's filter (mix -> BiquadFilterNode -> analyser): with one attached, sg_stream_push filters each channel's new
+ * chunk on the device, in place, before framing it.  NULL detaches the filter and drops its state.  The first attach
+ * starts from zero state; changing the parameters while attached keeps the state (an AudioParam change between render
+ * quanta, what dragging in draw mode does).  sg_stream_reset zeroes the state and keeps the parameters.  Works with any
+ * cfg.output, with or without a sonogram history.  Errors as sg_biquad_coefficients. */
+int sg_stream_set_filter(sg_stream* s, const sg_biquad_params* p);
+
 /* ------------------------------------------------------------------ PCM ingestion ---------- */
 /* The step in front of the path: the reference hands an encoded file to the browser,
  * context.decodeAudioData(request.response, buffer => ...) (util/util.js:9-17), plays the resulting

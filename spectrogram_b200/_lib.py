@@ -63,6 +63,15 @@ class PcmInfo(C.Structure):
                 ("frames", C.c_int64), ("data_offset", C.c_int64)]
 
 
+class BiquadParams(C.Structure):
+    """``sg_biquad_params``."""
+
+    _fields_ = [("type", C.c_int32), ("sample_rate", C.c_double), ("frequency", C.c_double), ("q", C.c_double),
+                ("gain", C.c_double), ("detune", C.c_double)]
+
+
+BIQUAD_TYPES = ("lowpass", "highpass", "bandpass", "lowshelf", "highshelf", "peaking", "notch", "allpass")
+
 # name -> (restype, argtypes); every symbol include/sgcore.h declares
 SIGNATURES = {
     "sg_last_error": (C.c_char_p, []),
@@ -113,6 +122,12 @@ SIGNATURES = {
     "sg_stream_history_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "sg_stream_history_read": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "sg_stream_view": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "sg_biquad_coefficients": (C.c_int, [C.POINTER(BiquadParams), C.c_void_p]),
+    "sg_biquad_filter": (C.c_int, [C.c_void_p, C.POINTER(BiquadParams), C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                   C.c_void_p]),
+    "sg_biquad_filter_device": (C.c_int, [C.c_void_p, C.POINTER(BiquadParams), C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
+                                          C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "sg_stream_set_filter": (C.c_int, [C.c_void_p, C.POINTER(BiquadParams)]),
     "sg_pcm_sample_bytes": (C.c_int, [C.c_int]),
     "sg_pcm_num_planes": (C.c_int, [C.POINTER(PcmInfo), C.c_int]),
     "sg_wav_parse": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(PcmInfo)]),

@@ -272,6 +272,16 @@ class Engine:
         L.check(self._lib.sg_stft_batch_device(self.handle, C.c_void_p(pcm_ptr), n_clips, clip_len, clip_stride,
                                                C.byref(cfg), C.c_void_p(out_ptr), C.c_void_p(stream)))
 
+    def biquad_device(self, node, in_ptr: int, n_channels: int, length: int, in_stride: int, out_ptr: int,
+                      out_stride: int, state_ptr: int = 0, stream: int = 0) -> None:
+        """``sg_biquad_filter_device`` with ``node``'s parameters (a BiquadFilterNode; its own state is not used):
+        float32 channels at ``in_ptr + c*in_stride`` -> ``out_ptr + c*out_stride``, in place when the pointers and
+        strides are equal.  ``state_ptr``: device [n_channels][4] float64 carried state, or 0.  Asynchronous."""
+        p = node.params()
+        L.check(self._lib.sg_biquad_filter_device(self.handle, C.byref(p), C.c_void_p(in_ptr), n_channels, length,
+                                                  in_stride, C.c_void_p(out_ptr), out_stride,
+                                                  C.c_void_p(state_ptr or None), C.c_void_p(stream)))
+
 
 _default_engines: dict[int, Engine] = {}
 _default_lock = threading.Lock()
@@ -355,15 +365,23 @@ class PinnedArray:
             pass
 
 
+def _param_key(p: L.BiquadParams) -> tuple:
+    return (p.type, p.sample_rate, p.frequency, p.q, p.gain, p.detune)
+
+
 class StreamBank:
     """``sg_stream``: n_channels analysers advanced in lock step (BASELINE config 5).
 
     ``history_rows``: keep a sonogram history per channel on the device (``sg_stream_set_history``) -- what a
     ``SonogramRing(bins, history_rows)`` fed every push's byte rows would hold -- so ``view()`` renders every channel's
-    picture in one launch without the rows crossing PCIe twice.  Needs ``output="u8"``."""
+    picture in one launch without the rows crossing PCIe twice.  Needs ``output="u8"``.
+
+    ``filter``: a BiquadFilterNode in front of every channel's analyser (``sg_stream_set_filter``; the reference's draw
+    mode).  The bank keeps the filter state on the device and re-sends the node's parameters before a push when they
+    changed since the last one; the node's own ``process`` state is not used."""
 
     def __init__(self, n_channels: int, opts: Options, max_chunk: int | None = None, engine: Engine | None = None,
-                 history_rows: int | None = None):
+                 history_rows: int | None = None, filter=None):
         self.engine = engine or default_engine(0)
         self._lib = L.load()
         self.opts = opts
@@ -374,8 +392,35 @@ class StreamBank:
         h = C.c_void_p()
         L.check(self._lib.sg_stream_create(self.engine.handle, self.n_channels, C.byref(cfg), self.max_chunk, C.byref(h)))
         self._h = h
+        self._filter = None
+        self._filter_sent = None
         if history_rows is not None:
             self.set_history(history_rows)
+        if filter is not None:
+            self.set_filter(filter)
+
+    # -- biquad filter in front of the analysers ---------------------------------------------------
+    def set_filter(self, node) -> None:
+        """Attach ``node`` (a BiquadFilterNode) or detach with None.  The first attach starts from zero state; a new
+        node or new parameters while attached keep it; detaching drops it."""
+        if node is None:
+            L.check(self._lib.sg_stream_set_filter(self._h, None))
+            self._filter = self._filter_sent = None
+            return
+        p = node.params()
+        L.check(self._lib.sg_stream_set_filter(self._h, C.byref(p)))
+        self._filter, self._filter_sent = node, _param_key(p)
+
+    @property
+    def filter(self):
+        return self._filter
+
+    def _sync_filter(self) -> None:
+        if self._filter is not None:
+            p = self._filter.params()
+            if _param_key(p) != self._filter_sent:
+                L.check(self._lib.sg_stream_set_filter(self._h, C.byref(p)))
+                self._filter_sent = _param_key(p)
 
     def push(self, chunk, out=None, out_rgba=None, want_rgba: bool = False):
         x = np.ascontiguousarray(chunk, dtype=np.float32)
@@ -388,6 +433,7 @@ class StreamBank:
             out = np.empty(shape, dtype=dt)
         if want_rgba and out_rgba is None:
             out_rgba = np.empty((self.n_channels, frames, self._cfg.n_fft // 2, 4), dtype=np.uint8)
+        self._sync_filter()
         L.check(self._lib.sg_stream_push(self._h, x.ctypes.data, chunk_len, out.ctypes.data,
                                          out_rgba.ctypes.data if out_rgba is not None else None))
         return (out, out_rgba) if out_rgba is not None else out
@@ -397,6 +443,7 @@ class StreamBank:
         x = np.ascontiguousarray(chunk, dtype=np.float32)
         if x.ndim != 2 or x.shape[0] != self.n_channels:
             raise TypeError("chunk must be [n_channels, chunk_len]")
+        self._sync_filter()
         L.check(self._lib.sg_stream_push(self._h, x.ctypes.data, x.shape[1], None, None))
 
     def reset(self):

@@ -124,6 +124,9 @@ int launch_pcm_ingest(int format, const PcmGeom& g, long long n_clips, const Pcm
 // tu_resample.cu: PCM ingestion + polyphase resampling (kernel_resample.cuh); tile_out and tiles are set by the launcher
 struct RsGeom;
 int launch_pcm_resample(int format, RsGeom g, long long n_clips, const PcmMix& m, cudaStream_t st);
+// tu_biquad.cu: biquad filter (kernel_biquad.cuh)
+struct BqArgs;
+int launch_biquad(const BqArgs& a, cudaStream_t st, int* launches);
 
 #ifdef SG_DEBUG
 int dbg_attach_w32x2p(const DbgState& st);

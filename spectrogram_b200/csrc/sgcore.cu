@@ -22,6 +22,7 @@
 #include "kernel_w32x2s.cuh"
 #include "kernel_pcm.cuh"
 #include "kernel_resample.cuh"
+#include "kernel_biquad.cuh"
 #include "plans.cuh"
 using sg::PcmMix; using sg::PcmGeom; using sg::kPcmMaxChannels; using sg::pcm_tile_frames; using sg::launch_pcm_ingest;
 using sg::RsGeom; using sg::launch_pcm_resample;
@@ -352,6 +353,7 @@ struct sg_engine {
   unsigned xs_epoch = 0;
   DevBuf d_raw[2];                   // interleaved PCM bytes in flight (sg_stft_pcm)
   std::map<std::pair<int, int>, RsTable> rs_tables;   // resampling filters by (up, down)
+  DevBuf bq_start, bq_agg, bq_io, bq_state;           // biquad filter: tile records (shared scratch), host-call staging
   PinBuf pin_in[2], pin_out[2];
   int64_t launches = 0;
   int kernel_variant = 0;            // 0 auto, 1 force generic smem kernel
@@ -857,6 +859,7 @@ int sg_engine_destroy(sg_engine* e) {
   e->lut_user.release(); e->scratch_mag.release(); e->scratch_state.release(); e->scratch_carry.release(); e->xs_carry.release(); e->xs_flags.release(); e->xs_state.release(); e->d_in.release(); e->d_out.release();
   e->d_raw[0].release(); e->d_raw[1].release();
   for (auto& kv : e->rs_tables) kv.second.taps.release();
+  e->bq_start.release(); e->bq_agg.release(); e->bq_io.release(); e->bq_state.release();
   for (int i = 0; i < 2; ++i) { e->pin_in[i].release(); e->pin_out[i].release(); }
   if (e->stream) cudaStreamDestroy(e->stream);
   if (e->s_h2d) cudaStreamDestroy(e->s_h2d);
@@ -1213,5 +1216,6 @@ int sg_stft_batch_multi(sg_engine* const* engines, int n_engines, const float* p
 }
 }  // extern "C"
 
+#include "sg_biquad.inl"
 #include "sg_objects.inl"
 #include "sg_pcm.inl"

@@ -152,6 +152,52 @@ function spectrogram(pcm, opts) {
 
 // opts.historyRows keeps a sonogram history per channel on the device: what a SonogramRing(bins, historyRows) fed
 // every push's byte rows would hold.  view() then draws every channel's picture in one launch (output 'u8' only).
+// BiquadFilterNode (W3C Web Audio), the filter the reference's draw mode puts in front of its analyser
+// (Player.setBandpassFrequency, UI/player.js): bandpass.type = 'bandpass'; bandpass.Q.value = 10;
+// bandpass.frequency.value = f.  process() filters on the GPU and carries the float64 state between calls.
+const BIQUAD_TYPES = ['lowpass', 'highpass', 'bandpass', 'lowshelf', 'highshelf', 'peaking', 'notch', 'allpass'];
+class AudioParam {
+  constructor(value) {
+    this.defaultValue = value;
+    this.value = value;
+  }
+}
+class BiquadFilterNode {
+  constructor(options) {
+    const o = options || {};
+    this.sampleRate = o.sampleRate || 48000;
+    this.channels = o.channels || 1;
+    this._device = o.device || 0;
+    this._type = 'lowpass';
+    this.frequency = new AudioParam(350);
+    this.Q = new AudioParam(1);
+    this.gain = new AudioParam(0);
+    this.detune = new AudioParam(0);
+    this._state = new Float64Array(4 * this.channels);   // [channel] {x1, x2, y1, y2}
+  }
+  get type() { return this._type; }
+  // WebIDL enum attribute: assigning a string outside the enum is ignored, not thrown
+  set type(value) { if (BIQUAD_TYPES.includes(value)) this._type = value; }
+  params() {
+    return { type: this._type, sampleRate: this.sampleRate, frequency: this.frequency.value, Q: this.Q.value,
+             gain: this.gain.value, detune: this.detune.value };
+  }
+  // normalised Float64Array [b0, b1, b2, a1, a2]
+  coefficients() {
+    const out = new Float64Array(5);
+    guard(native.biquadCoefficients)(this.params(), out);
+    return out;
+  }
+  // samples: Float32Array [channel][n]; returns (or fills `out`) the filtered samples
+  process(samples, out) {
+    const len = wholeNumber(samples.length / this.channels, 'samples.length / channels');
+    const dst = out || new Float32Array(samples.length);
+    guard(native.biquadFilter)(engineFor(this._device), this.params(), samples, this.channels, len, this._state, dst);
+    return dst;
+  }
+  reset() { this._state.fill(0); }
+}
+
 class StreamBank {
   constructor(nChannels, opts, maxChunk) {
     this.opts = Object.assign({ fftSize: 1024, hop: 128, output: 'u8' }, opts || {});
@@ -160,11 +206,27 @@ class StreamBank {
     this._h = guard(native.streamCreate)(engineFor(this.opts.device || 0), nChannels, this.opts, this.maxChunk);
     own(this, native.streamDestroy, this._h);
     if (this.opts.historyRows) this.setHistory(this.opts.historyRows);
+    this._filter = null;
+    if (this.opts.filter) this.setFilter(this.opts.filter);
+  }
+  // a BiquadFilterNode in front of every channel's analyser (the draw mode's bandpass), or null to detach it.  The bank
+  // keeps the filter state on the device; the node's parameters are re-sent before a push when they have changed.
+  setFilter(node) {
+    const p = node ? node.params() : null;
+    guard(native.streamSetFilter)(this._h, p);
+    this._filter = node || null;
+    this._filterSent = p && JSON.stringify(p);
+  }
+  _syncFilter() {
+    if (!this._filter) return;
+    const p = this._filter.params(), key = JSON.stringify(p);
+    if (key !== this._filterSent) { guard(native.streamSetFilter)(this._h, p); this._filterSent = key; }
   }
   // chunk: Float32Array [channel][chunkLen]; out: typed array [channel][chunkLen/hop][bins], or undefined when a
   // history is attached and only the pictures are wanted (no rows come back to the host)
   push(chunk, out, outRgba) {
     const chunkLen = wholeNumber(chunk.length / this.nChannels, 'chunk.length / nChannels');
+    this._syncFilter();
     guard(native.streamPush)(this._h, chunk, chunkLen, out, outRgba);
   }
   // attach an empty history of `rows` rows per channel (texture zero, yoffset 0); 0 detaches it
@@ -312,6 +374,9 @@ module.exports = {
   createAnalyser: (options) => new AnalyserNode(options),
   spectrogram,
   StreamBank,
+  BiquadFilterNode,
+  AudioParam,
+  createBiquadFilter: (options) => new BiquadFilterNode(options),
   SonogramRing,
   AudioBuffer,
   decodeAudioData,

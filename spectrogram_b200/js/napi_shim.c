@@ -14,6 +14,7 @@
  * (node_api_min.h) and exercised by tests/napi_host/fake_napi_host.c, a C host that supplies the
  * napi_* symbols.  Under real Node the same object file loads unchanged.
  */
+#include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -543,6 +544,97 @@ static napi_value js_stream_destroy(napi_env env, napi_callback_info info) {
   return undefined_of(env);
 }
 
+/* ---------------------------------------------------------------- biquad filter */
+static const char* const kBiquadNames[8] = {"lowpass", "highpass", "bandpass", "lowshelf", "highshelf", "peaking", "notch", "allpass"};
+
+/* {type, sampleRate, frequency, Q, gain, detune} -> sg_biquad_params; absent members take the BiquadFilterNode defaults
+ * (lowpass, 48000, 350, 1, 0, 0).  Returns 0 and leaves a TypeError pending on a non-object or an unknown type (the JS
+ * facade never sends one: it ignores such assignments, as WebIDL does for an enum attribute). */
+static int parse_biquad(napi_env env, napi_value obj, sg_biquad_params* p) {
+  napi_valuetype t;
+  char s[32];
+  int i;
+  p->type = SG_BIQUAD_LOWPASS; p->sample_rate = 48000.0; p->frequency = 350.0; p->q = 1.0; p->gain = 0.0; p->detune = 0.0;
+  if (napi_typeof(env, obj, &t) != napi_ok || t != napi_object) {
+    type_error(env, "filter parameters must be an object");
+    return 0;
+  }
+  prop_double(env, obj, "sampleRate", &p->sample_rate);
+  prop_double(env, obj, "frequency", &p->frequency);
+  prop_double(env, obj, "Q", &p->q);
+  prop_double(env, obj, "gain", &p->gain);
+  prop_double(env, obj, "detune", &p->detune);
+  if (prop_string(env, obj, "type", s, sizeof s)) {
+    for (i = 0; i < 8 && strcmp(s, kBiquadNames[i]); ++i) {}
+    if (i == 8) {
+      type_error(env, "unknown biquad type");
+      return 0;
+    }
+    p->type = i;
+  }
+  return 1;
+}
+
+/* biquadCoefficients(params, out: Float64Array >= 5) -> normalised b0, b1, b2, a1, a2 */
+static napi_value js_biquad_coefficients(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  sg_biquad_params p;
+  void* out;
+  size_t n;
+  int rc;
+  if (get_args(env, info, argv) < 2) return type_error(env, "biquadCoefficients(params, out)");
+  if (!parse_biquad(env, argv[0], &p)) return undefined_of(env);
+  if (!get_typed(env, argv[1], napi_float64_array, &out, &n) || n < 5) return type_error(env, "out must be a Float64Array of 5 entries");
+  rc = sg_biquad_coefficients(&p, (double*)out);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
+/* biquadFilter(engine, params, samples: Float32Array [channels][len], channels, len, state: Float64Array [channels][4] |
+ * undefined, out: Float32Array [channels][len]) */
+static napi_value js_biquad_filter(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  sg_biquad_params p;
+  void *e, *in, *out, *state = NULL;
+  size_t in_n, out_n, state_n = 0;
+  int64_t channels, len;
+  uint64_t need;
+  int rc;
+  if (get_args(env, info, argv) < 7 || !get_external(env, argv[0], &e))
+    return type_error(env, "biquadFilter(engine, params, samples, channels, len, state, out)");
+  if (!parse_biquad(env, argv[1], &p)) return undefined_of(env);
+  if (!get_typed(env, argv[2], napi_float32_array, &in, &in_n)) return type_error(env, "samples must be a Float32Array");
+  if (napi_get_value_int64(env, argv[3], &channels) != napi_ok || napi_get_value_int64(env, argv[4], &len) != napi_ok ||
+      channels < 0 || len < 0)
+    return type_error(env, "channels and len must be non-negative integers");
+  if (!is_undefined(env, argv[5]) && !get_typed(env, argv[5], napi_float64_array, &state, &state_n))
+    return type_error(env, "state must be a Float64Array or undefined");
+  if (!get_typed(env, argv[6], napi_float32_array, &out, &out_n)) return type_error(env, "out must be a Float32Array");
+  /* the core reads and writes channels * len samples and channels * 4 state values: check before any pointer goes over */
+  if (channels > 0 && (uint64_t)len > UINT64_MAX / (uint64_t)channels) return type_error(env, "channels * len overflows");
+  need = (uint64_t)channels * (uint64_t)len;
+  if ((uint64_t)in_n < need) return type_error(env, "samples is shorter than channels * len");
+  if ((uint64_t)out_n < need) return type_error(env, "out is shorter than channels * len");
+  if (state && (uint64_t)state_n < 4 * (uint64_t)channels) return type_error(env, "state is shorter than channels * 4");
+  rc = sg_biquad_filter((sg_engine*)e, &p, (const float*)in, channels, len, (double*)state, (float*)out);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
+/* streamSetFilter(stream, params | null | undefined): attach or retune the bank's filter; null detaches it */
+static napi_value js_stream_set_filter(napi_env env, napi_callback_info info) {
+  napi_value argv[MAX_ARGS];
+  sg_biquad_params p;
+  void* s;
+  int rc, channels = 0;
+  if (get_args(env, info, argv) < 2 || !get_external(env, argv[0], &s)) return type_error(env, "streamSetFilter(stream, params)");
+  if (sg_stream_info((sg_stream*)s, &channels, NULL, NULL, NULL, NULL) != SG_OK) return type_error(env, "stream expected");
+  if (!is_undefined(env, argv[1]) && !parse_biquad(env, argv[1], &p)) return undefined_of(env);
+  rc = sg_stream_set_filter((sg_stream*)s, is_undefined(env, argv[1]) ? NULL : &p);
+  if (rc != SG_OK) return throw_status(env, rc);
+  return undefined_of(env);
+}
+
 /* ---------------------------------------------------------------- sonogram ring + view */
 /* ringCreate(engine, bins, rows): the reference's bins x 256 byte texture (3D/visualizer.js:301-329) */
 static napi_value js_ring_create(napi_env env, napi_callback_info info) {
@@ -829,6 +921,9 @@ napi_value napi_register_module_v1(napi_env env, napi_value exports) {
   export_fn(env, exports, "resampleNumFrames", js_resample_num_frames);
   export_fn(env, exports, "pcmDecodeResampled", js_pcm_decode_resampled);
   export_fn(env, exports, "stftPcmResampled", js_stft_pcm_resampled);
+  export_fn(env, exports, "biquadCoefficients", js_biquad_coefficients);
+  export_fn(env, exports, "biquadFilter", js_biquad_filter);
+  export_fn(env, exports, "streamSetFilter", js_stream_set_filter);
   return exports;
 }
 

@@ -59,6 +59,12 @@ for n_fft, clips in ((4096, 160), (1024, 160), (512, 40), (256, 3)):
     eng.spectrogram(big[:clips], sg.Options(fftSize=n_fft, hop=n_fft // 4, smoothingTimeConstant=0.8))
     seen.add(eng.last_kernel)
 eng.set_kernel_variant(0)
+# the biquad filter: one tile per channel (one launch), and channels of several tiles (tile aggregates, carry scan, emit)
+bq = sg.BiquadFilterNode(eng, channels=3)
+bq.type = "bandpass"
+for n in (300, 3 * 4096 + 77):
+    bq.process(x[:, :n] if n <= x.shape[1] else np.tile(x, (1, 2))[:, :n])
+    seen.add(eng.last_kernel)
 lib = sg._lib.load()
 if hasattr(lib, "sg_debug_counts"):
     counts = (C.c_ulonglong * 16)()
