@@ -202,7 +202,8 @@ int sg_stream_reset(sg_stream* s); /* zero history and smoothing state, and clea
  * out: host [n_channels][chunk_len/hop][bins] elements of cfg.output.  It may be NULL when a
  * sonogram history is attached (sg_stream_set_history): the rows then only land in the history.
  * out_rgba (may be NULL): additionally host [n_channels][chunk_len/hop][bins] RGBA8 through the
- * colour LUT (only when cfg.output == SG_OUT_U8, and only with out).  Synchronous: returns when
+ * colour LUT, cfg.colormap or the reference's when it is NULL (only when cfg.output == SG_OUT_U8,
+ * and only with out).  Synchronous: returns when
  * both are filled and the history holds the new rows. */
 int sg_stream_push(sg_stream* s, const float* chunk, int chunk_len, void* out, uint32_t* out_rgba);
 int64_t sg_stream_frames_emitted(const sg_stream* s); /* per channel */

@@ -13,20 +13,23 @@ namespace sg {
 // the initial X^ and written back with the final one (so chunks of one clip can be chained, and
 // the streaming objects keep it across calls).  Arithmetic as Chromium: double, stored as float.
 // HBM-bound: 4 B read + elem B written per (frame, bin); coalesced across bins.
-// A non-finite magnitude (a frame with NaN / Inf samples, or |X|^2 overflowing float) enters the recurrence as 0 in
-// this two-kernel path -- the time-parallel form below needs finite inputs to stay linear -- so X^ decays over such a
-// frame; the fused kernel (kernel_w32x2s.cuh) applies [SPEC]'s "non-finite X^ -> 0" literally and restarts from 0.
+// [SPEC] "non-finite X^ -> 0": the frame kernels write the magnitudes of a frame with a NaN / Inf sample as 0, which
+// the recurrence cannot tell from silence, so `poison` ([n_clips][frames], poison_flags_kernel) names those frames and
+// the state restarts from 0 there, as in the fused kernels.  poison == nullptr: no frame is poisoned (the AnalyserNode
+// object, whose non-finite magnitudes enter the recurrence as 0).  A magnitude that is itself non-finite (|X|^2
+// overflowing float) enters as 0.
 template <int OUT>
 __global__ void __launch_bounds__(256)
 smooth_emit_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* __restrict__ out,
                    float* __restrict__ state, long long n_clips, long long frames, int bins, double tau,
-                   Epilogue ep) {
+                   Epilogue ep, const uint8_t* __restrict__ poison) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= n_clips * bins) return;
   const long long clip = idx / bins;
   const int b = (int)(idx - clip * bins);
   const float* __restrict__ m = mags + clip * frames * bins + b;
   typename OutElem<OUT>::type* __restrict__ o = out + clip * frames * bins + b;
+  const uint8_t* __restrict__ pz = poison ? poison + clip * frames : nullptr;
   float s = state[idx];
   const double k1 = 1.0 - tau;
   long long t = 0;
@@ -37,14 +40,33 @@ smooth_emit_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* 
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       s = finite_or_zero((float)(tau * (double)s + k1 * (double)v[u]));
+      if (pz && __ldg(pz + t + u)) s = 0.f;
       o[(t + u) * bins] = emit_mag<OUT>(s, ep);
     }
   }
   for (; t < frames; ++t) {
     s = finite_or_zero((float)(tau * (double)s + k1 * (double)finite_or_zero(__ldg(m + t * bins))));
+    if (pz && __ldg(pz + t)) s = 0.f;
     o[t * bins] = emit_mag<OUT>(s, ep);
   }
   state[idx] = s;
+}
+
+// poison[clip][t] = 1 when frame t of the clip holds a NaN / Inf sample (samples outside the clip are the zero
+// history): what smooth_emit_kernel and smooth_scan_kernel restart the state on.  One warp per frame, coalesced loads
+// (a sample is read by n_fft / hop frames; the overlap comes from L2).
+__global__ void __launch_bounds__(256) poison_flags_kernel(FrameGeom g, uint8_t* __restrict__ poison) {
+  const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (w >= g.total_frames) return;     // (whole warps)
+  const long long clip = w / g.frames_per_clip, t = w - clip * g.frames_per_clip;
+  const float* __restrict__ x = g.pcm + clip * g.clip_stride;
+  const long long s0 = g.start0 + t * g.hop;
+  const long long lo = s0 > 0 ? s0 : 0, hi = s0 + g.n_fft < g.clip_len ? s0 + g.n_fft : g.clip_len;
+  bool bad = false;
+  for (long long i = lo + lane; i < hi; i += 32) bad |= !(fabsf(__ldg(x + i)) <= 3.4028235e38f);
+  bad = __any_sync(0xffffffffu, bad);
+  if (lane == 0) poison[w] = bad ? 1 : 0;
 }
 
 // ---- time-parallel form of the same recurrence for long clips with few (clip, bin) pairs, ONE kernel ---------------
@@ -57,9 +79,11 @@ smooth_emit_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* 
 //       in L1/L2).
 // The three phases are grid-stride loops of one cooperative launch separated by grid barriers (the grid is sized to
 // be co-resident), so a two-channel clip costs one launch after its frame kernel instead of three.
-// Inputs are finite (the frame kernels map non-finite magnitudes to 0), so the [SPEC] non-finite rule cannot fire
-// inside the sums; phase (C) still applies it per frame like the sequential kernel.  The carried state differs from
-// the sequential kernel's by float rounding of the chunk sums (a few ulp): tests/test_gpu_parity.py compares the two.
+// A poisoned frame (see smooth_emit_kernel) restarts the state: (A) restarts its local sum there and records the
+// restart in the sign bit of the chunk's carry (the sums are never negative, so -0.0 still says so), (B) gives such a
+// chunk decay 0 -- its scan composes affine steps s' = d_j s + l_j with d_j = dec or 0 -- and (C) restarts per frame
+// like the sequential kernel.  The carried state differs from the sequential kernel's by float rounding of the chunk
+// sums (a few ulp): tests/test_gpu_parity.py compares the two.
 // carry: [n_clips][bins][n_chunks] float (chunk fastest: phase B reads a bin's chunks coalesced).
 struct ScanGeom {
   long long n_clips, frames, n_chunks;
@@ -70,7 +94,8 @@ struct ScanGeom {
 template <int OUT>
 __global__ void __launch_bounds__(256)
 smooth_scan_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* __restrict__ out,
-                   float* __restrict__ state, float* __restrict__ carry, ScanGeom sg_, Epilogue ep) {
+                   float* __restrict__ state, float* __restrict__ carry, ScanGeom sg_, Epilogue ep,
+                   const uint8_t* __restrict__ poison) {
   cooperative_groups::grid_group grid = cooperative_groups::this_grid();
   const long long n_clips = sg_.n_clips, frames = sg_.frames, n_chunks = sg_.n_chunks;
   const int bins = sg_.bins, chunk = sg_.chunk;
@@ -84,7 +109,9 @@ smooth_scan_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* 
     if (j + 1 == n_chunks) continue;          // the last chunk is nobody's predecessor
     const long long t0 = j * chunk, t1 = min(frames, t0 + (long long)chunk);
     const float* __restrict__ m = mags + clip * frames * bins + b;
+    const uint8_t* __restrict__ pz = poison ? poison + clip * frames : nullptr;
     double s = 0.0;
+    bool restart = false;
     long long t = t0;
     // the loads do not depend on the recurrence: eight in flight per thread, then eight dependent updates
     for (; t + 8 <= t1; t += 8) {
@@ -92,35 +119,44 @@ smooth_scan_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* 
 #pragma unroll
       for (int u = 0; u < 8; ++u) v[u] = finite_or_zero(__ldg(m + (t + u) * bins));
 #pragma unroll
-      for (int u = 0; u < 8; ++u) s = tau * s + k1 * (double)v[u];
+      for (int u = 0; u < 8; ++u) {
+        s = tau * s + k1 * (double)v[u];
+        if (pz && __ldg(pz + t + u)) { s = 0.0; restart = true; }
+      }
     }
-    for (; t < t1; ++t) s = tau * s + k1 * (double)finite_or_zero(__ldg(m + t * bins));
-    carry[(clip * bins + b) * n_chunks + j] = (float)s;
+    for (; t < t1; ++t) {
+      s = tau * s + k1 * (double)finite_or_zero(__ldg(m + t * bins));
+      if (pz && __ldg(pz + t)) { s = 0.0; restart = true; }
+    }
+    const float local = (float)s;
+    carry[(clip * bins + b) * n_chunks + j] = restart ? -local : local;
   }
   grid.sync();
   // ---- (B) carry[j] <- state at the START of chunk j (in place); state[clip][bin] holds the clip's initial state
   {
     const int lane = threadIdx.x & 31;
     const double dec = pow(tau, (double)chunk);   // every chunk but the last is full, and the last one's decay is unused
-    double dpow[5];                               // dec^(2^k)
-    dpow[0] = dec;
-#pragma unroll
-    for (int k = 1; k < 5; ++k) dpow[k] = dpow[k - 1] * dpow[k - 1];
-    const double dec_lane = pow(dec, (double)lane), dec32 = dpow[4] * dpow[4];
     for (long long w = tid >> 5; w < n_clips * bins; w += nthreads >> 5) {
       float* __restrict__ c = carry + w * n_chunks;
       double s = (double)state[w];               // state at the start of the current 32-chunk segment
       for (long long j0 = 0; j0 < n_chunks; j0 += 32) {
         const long long j = j0 + lane;
-        double y = j + 1 < n_chunks ? (double)__ldcg(c + j) : 0.0;   // inclusive decayed prefix sum of the locals
+        // chunk j maps the state at its start to d * s + y; the last chunk (nobody's predecessor) and lanes past the
+        // end are the identity.  Inclusive scan of the composition (d, y) then (d', y') = (d d', d' y + y').
+        double d = 1.0, y = 0.0;
+        if (j + 1 < n_chunks) {
+          const float v = __ldcg(c + j);
+          d = signbit(v) ? 0.0 : dec;
+          y = (double)fabsf(v);
+        }
 #pragma unroll
         for (int k = 0; k < 5; ++k) {
-          const double up = __shfl_up_sync(0xffffffffu, y, 1 << k);
-          if (lane >= (1 << k)) y = fma(dpow[k], up, y);
+          const double up_d = __shfl_up_sync(0xffffffffu, d, 1 << k), up_y = __shfl_up_sync(0xffffffffu, y, 1 << k);
+          if (lane >= (1 << k)) { y = fma(d, up_y, y); d *= up_d; }
         }
-        const double prev = __shfl_up_sync(0xffffffffu, y, 1);  // sum of the locals before this chunk
-        if (j < n_chunks) c[j] = (float)(fma(dec_lane, s, lane ? prev : 0.0));
-        s = fma(dec32, s, __shfl_sync(0xffffffffu, y, 31));
+        const double prev_d = __shfl_up_sync(0xffffffffu, d, 1), prev_y = __shfl_up_sync(0xffffffffu, y, 1);
+        if (j < n_chunks) c[j] = (float)(lane ? fma(prev_d, s, prev_y) : s);   // the state at the start of chunk j
+        s = fma(__shfl_sync(0xffffffffu, d, 31), s, __shfl_sync(0xffffffffu, y, 31));
       }
     }
   }
@@ -132,6 +168,7 @@ smooth_scan_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* 
     const long long t0 = j * chunk, t1 = min(frames, t0 + (long long)chunk);
     const float* __restrict__ m = mags + clip * frames * bins + b;
     typename OutElem<OUT>::type* __restrict__ o = out + clip * frames * bins + b;
+    const uint8_t* __restrict__ pz = poison ? poison + clip * frames : nullptr;
     float s = __ldcg(carry + (clip * bins + b) * n_chunks + j);
     long long t = t0;
     for (; t + 8 <= t1; t += 8) {
@@ -141,11 +178,13 @@ smooth_scan_kernel(const float* __restrict__ mags, typename OutElem<OUT>::type* 
 #pragma unroll
       for (int u = 0; u < 8; ++u) {
         s = finite_or_zero((float)(tau * (double)s + k1 * (double)v[u]));
+        if (pz && __ldg(pz + t + u)) s = 0.f;
         o[(t + u) * bins] = emit_mag<OUT>(s, ep);
       }
     }
     for (; t < t1; ++t) {
       s = finite_or_zero((float)(tau * (double)s + k1 * (double)finite_or_zero(__ldg(m + t * bins))));
+      if (pz && __ldg(pz + t)) s = 0.f;
       o[t * bins] = emit_mag<OUT>(s, ep);
     }
     if (j == n_chunks - 1) state[clip * bins + b] = s;

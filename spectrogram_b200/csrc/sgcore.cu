@@ -348,7 +348,7 @@ struct sg_engine {
   std::map<PlanKey, Plan> plans;
   uint32_t* lut_ref = nullptr;       // device, reference colour map
   DevBuf lut_user;                   // device copy of cfg.colormap
-  DevBuf scratch_mag, scratch_state, scratch_carry, d_in, d_out;
+  DevBuf scratch_mag, scratch_state, scratch_carry, scratch_poison, d_in, d_out;
   DevBuf xs_carry, xs_flags, xs_state;         // fused-smoothing kernel: per-segment carry vectors and their ready flags
   unsigned xs_epoch = 0;
   DevBuf d_raw[2];                   // interleaved PCM bytes in flight (sg_stft_pcm)
@@ -483,7 +483,7 @@ int launch_frames(sg_engine* e, const Plan& pl, const sg::FrameGeom& g, const sg
 
 template <int OUT>
 int launch_smooth_t(sg_engine* e, const float* mags, void* out, float* state, long long n_clips, long long frames,
-                    int bins, double tau, const sg::Epilogue& ep, cudaStream_t st) {
+                    int bins, double tau, const sg::Epilogue& ep, const uint8_t* poison, cudaStream_t st) {
   using T = typename sg::OutElem<OUT>::type;
   const long long n = n_clips * bins;
   if (n <= 0 || frames <= 0) return SG_OK;
@@ -504,27 +504,38 @@ int launch_smooth_t(sg_engine* e, const float* mags, void* out, float* state, lo
     sg::ScanGeom sgm{n_clips, frames, n_chunks, bins, chunk, tau};
     T* out_t = (T*)out;
     sg::Epilogue ep_c = ep;
-    void* args[] = {(void*)&mags, (void*)&out_t, (void*)&state, (void*)&carry, (void*)&sgm, (void*)&ep_c};
+    void* args[] = {(void*)&mags, (void*)&out_t, (void*)&state, (void*)&carry, (void*)&sgm, (void*)&ep_c, (void*)&poison};
     SG_CUDA(cudaLaunchCooperativeKernel((const void*)sg::smooth_scan_kernel<OUT>, dim3(grid), dim3(256), args, 0, st));
     e->launches++;
     SG_CUDA(cudaGetLastError());
     return SG_OK;
   }
   sg::smooth_emit_kernel<OUT><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(mags, (T*)out, state, n_clips, frames,
-                                                                          bins, tau, ep);
+                                                                          bins, tau, ep, poison);
   e->launches++;
   SG_CUDA(cudaGetLastError());
   return SG_OK;
 }
 
 int launch_smooth(sg_engine* e, int out_kind, const float* mags, void* out, float* state, long long n_clips,
-                  long long frames, int bins, double tau, const sg::Epilogue& ep, cudaStream_t st) {
+                  long long frames, int bins, double tau, const sg::Epilogue& ep, const uint8_t* poison, cudaStream_t st) {
   switch (out_kind) {
-    case SG_OUT_U8: return launch_smooth_t<sg::kOutU8>(e, mags, out, state, n_clips, frames, bins, tau, ep, st);
-    case SG_OUT_F32_DB: return launch_smooth_t<sg::kOutF32Db>(e, mags, out, state, n_clips, frames, bins, tau, ep, st);
-    case SG_OUT_RGBA8: return launch_smooth_t<sg::kOutRgba8>(e, mags, out, state, n_clips, frames, bins, tau, ep, st);
-    default: return launch_smooth_t<sg::kOutF32Mag>(e, mags, out, state, n_clips, frames, bins, tau, ep, st);
+    case SG_OUT_U8: return launch_smooth_t<sg::kOutU8>(e, mags, out, state, n_clips, frames, bins, tau, ep, poison, st);
+    case SG_OUT_F32_DB: return launch_smooth_t<sg::kOutF32Db>(e, mags, out, state, n_clips, frames, bins, tau, ep, poison, st);
+    case SG_OUT_RGBA8: return launch_smooth_t<sg::kOutRgba8>(e, mags, out, state, n_clips, frames, bins, tau, ep, poison, st);
+    default: return launch_smooth_t<sg::kOutF32Mag>(e, mags, out, state, n_clips, frames, bins, tau, ep, poison, st);
   }
+}
+
+// the frames of `g` that hold a NaN / Inf sample, [clip][frame] bytes in the engine's scratch: the two-kernel path's
+// recurrence restarts there ([SPEC] "non-finite X^ -> 0"; the frame kernel has already written their magnitudes as 0)
+int launch_poison(sg_engine* e, const sg::FrameGeom& g, cudaStream_t st, const uint8_t** out) {
+  SG_TRY(e->scratch_poison.reserve((size_t)g.total_frames));
+  sg::poison_flags_kernel<<<(unsigned)((g.total_frames * 32 + 255) / 256), 256, 0, st>>>(g, (uint8_t*)e->scratch_poison.p);
+  e->launches++;
+  SG_CUDA(cudaGetLastError());
+  *out = (const uint8_t*)e->scratch_poison.p;
+  return SG_OK;
 }
 
 // tau > 0 at n_fft 2048 / hop 512 or 256: the recurrence fused into the frame-pair kernel (kernel_w32x2s.cuh), one launch,
@@ -681,8 +692,8 @@ int launch_fused_smoothing(sg_engine* e, const Plan& pl, const sg_stft_config& c
 }
 
 // One launch group over `n_clips` clips x frames [t0, t0+nframes) of each clip.
-// tau == 0: a single fused kernel.  tau > 0: frame kernel -> linear magnitudes (scratch) ->
-// recurrence + dB/byte kernel, chained through `state` ([n_clips][bins]).
+// tau == 0: a single fused kernel.  tau > 0: a fused smoothing kernel, or the frames' non-finite flags, the frame
+// kernel -> linear magnitudes (scratch) and the recurrence + dB/byte kernel, chained through `state` ([n_clips][bins]).
 int run_range(sg_engine* e, const Plan& pl, const sg_stft_config& cfg, const float* pcm_dev, long long n_clips,
               long long clip_len, long long clip_stride, long long t0, long long nframes, long long frames_total,
               void* out_dev, float* state, const uint32_t* lut, cudaStream_t st) {
@@ -725,10 +736,12 @@ int run_range(sg_engine* e, const Plan& pl, const sg_stft_config& cfg, const flo
     for (long long c0 = 0; c0 < n_clips; c0 += group) {
       const long long nc = std::min(group, n_clips - c0);
       sg::FrameGeom g{pcm_dev + c0 * clip_stride, clip_len, clip_stride, nframes, nc * nframes, start0, cfg.n_fft, cfg.hop};
+      const uint8_t* poison;
+      SG_TRY(launch_poison(e, g, st, &poison));
       SG_TRY(launch_frames(e, pl, g, cfg, SG_OUT_F32_MAG, lut, e->scratch_mag.p, st));
       char* o = (char*)out_dev + (size_t)c0 * frames_total * bins * eb;
       SG_TRY(launch_smooth(e, cfg.output, (const float*)e->scratch_mag.p, o, state + c0 * bins, nc, nframes, bins,
-                           cfg.smoothing, ep, st));
+                           cfg.smoothing, ep, poison, st));
     }
     return SG_OK;
   }
@@ -738,10 +751,12 @@ int run_range(sg_engine* e, const Plan& pl, const sg_stft_config& cfg, const flo
     for (long long tt = 0; tt < nframes; tt += tile_frames) {
       const long long nt = std::min(tile_frames, nframes - tt);
       sg::FrameGeom g{pcm_dev + c * clip_stride, clip_len, clip_stride, nt, nt, start0 + tt * cfg.hop, cfg.n_fft, cfg.hop};
+      const uint8_t* poison;
+      SG_TRY(launch_poison(e, g, st, &poison));
       SG_TRY(launch_frames(e, pl, g, cfg, SG_OUT_F32_MAG, lut, e->scratch_mag.p, st));
       char* o = (char*)out_dev + ((size_t)c * frames_total + t0 + tt) * bins * eb;
       SG_TRY(launch_smooth(e, cfg.output, (const float*)e->scratch_mag.p, o, state + c * bins, 1, nt, bins, cfg.smoothing,
-                           ep, st));
+                           ep, poison, st));
     }
   return SG_OK;
 }
@@ -856,7 +871,7 @@ int sg_engine_destroy(sg_engine* e) {
   cudaDeviceSynchronize();
   for (auto& kv : e->plans) kv.second.release();
   cudaFree(e->lut_ref);
-  e->lut_user.release(); e->scratch_mag.release(); e->scratch_state.release(); e->scratch_carry.release(); e->xs_carry.release(); e->xs_flags.release(); e->xs_state.release(); e->d_in.release(); e->d_out.release();
+  e->lut_user.release(); e->scratch_mag.release(); e->scratch_state.release(); e->scratch_carry.release(); e->scratch_poison.release(); e->xs_carry.release(); e->xs_flags.release(); e->xs_state.release(); e->d_in.release(); e->d_out.release();
   e->d_raw[0].release(); e->d_raw[1].release();
   for (auto& kv : e->rs_tables) kv.second.taps.release();
   e->bq_start.release(); e->bq_agg.release(); e->bq_io.release(); e->bq_state.release();
