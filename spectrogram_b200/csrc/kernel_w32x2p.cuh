@@ -61,6 +61,41 @@ struct XpShape {
   static constexpr int kMaxRegs = NW <= 8 ? 255 : (65536 / (NW * 32)) / 8 * 8;
 };
 
+// Rotation.  A pair runs as three sections of similar FP32-pipe demand but different non-FMA content:
+//   A  window + pass 1 + exchange stores         B  exchange loads + pass 2 + mirror shuffles / selects
+//   C  untangle with the next pair's loads + epilogue
+// The warps of one scheduler (w, w + 4, w + 8: a rotation group) would otherwise reach the exchange, the shuffles and the
+// MUFU epilogue together and leave the FP32 pipe idle meanwhile.  Instead the group runs in steps separated by one group
+// barrier (ID 1 + group, NW / 4 warps): at step s, rank k (= w / 4) runs section (s + k) mod 3, so the ranks always sit in
+// different sections.  Rank k opens with xp_lead(k) barrier-only steps.  Every output but RGBA rotates (kRotate below).
+//
+// No warp may leave its group early: every warp of a group executes exactly xp_group_steps() barriers on the group's ID.
+// A warp's pairs are the frames 2 (block NW + w) + j * 2 grid NW (j >= 0) below total_frames, xp_warp_pairs() of them.
+// A warp with pairs spends xp_lead(k) steps before its first pair and 3 steps on each pair, xp_warp_steps() in all; the
+// group's count is the largest of its members', and every member spends the steps left over barrier-only (its tail, or
+// all of them for a warp without pairs).  Every input of xp_group_steps() is uniform over the CTA, so the members agree
+// on the count, and none of them runs short of it.  A group without pairs takes no step.
+__host__ __device__ constexpr int xp_lead(int rank) { return (3 - rank % 3) % 3; }
+__host__ __device__ inline long long xp_warp_pairs(long long total_frames, int grid, int nw, int block, int warp) {
+  const long long fa = 2 * ((long long)block * nw + warp), step = 2LL * grid * nw;
+  return fa < total_frames ? (total_frames - fa - 1) / step + 1 : 0;
+}
+__host__ __device__ inline long long xp_warp_steps(long long total_frames, int grid, int nw, int block, int warp) {
+  const long long n = xp_warp_pairs(total_frames, grid, nw, block, warp);
+  return n > 0 ? xp_lead(warp / 4) + 3 * n : 0;
+}
+__host__ __device__ inline long long xp_group_steps(long long total_frames, int grid, int nw, int block, int group) {
+  long long n = 0;
+  for (int warp = group; warp < nw; warp += 4) {
+    const long long s = xp_warp_steps(total_frames, grid, nw, block, warp);
+    n = s > n ? s : n;
+  }
+  return n;
+}
+__device__ __forceinline__ void xp_step_barrier(int group, int nw) {
+  asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "r"(nw / 4 * 32) : "memory");
+}
+
 // stage U (1..5) of pass 2: butterflies (i0, i0 + half), twiddle W_{2 half}^p * base
 template <int U>
 __device__ __forceinline__ void dit2_stage_gen(C2 (&a)[32], float2 base) {
@@ -118,7 +153,7 @@ __device__ __forceinline__ bool pair_is_fast(const FrameGeom& g, const PairP& p,
 // selects as PRMT instead of FSEL; 256: the mirrors through shared memory instead of shuffles)
 template <int OUT, int NW, int HOPJ = 8, int ABL = 0>   // hop = 64 * HOPJ samples: frame B's element j is element j + HOPJ of the lane
 __global__ void __launch_bounds__(NW * 32, 1) __maxnreg__(XpShape<NW>::kMaxRegs)
-stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::type* __restrict__ out, int stagger) {
+stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::type* __restrict__ out) {
   using T = typename OutElem<OUT>::type;
   constexpr int HOP = 64 * HOPJ, NLOAD = 32 + HOPJ, kLoadSteps = xp_load_steps<OUT, HOPJ>();
   extern __shared__ float4 smem_raw[];
@@ -144,14 +179,10 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
     for (int i = threadIdx.x; i < 16 * 32; i += blockDim.x) s_ut[i] = __ldg(pl.ut + i);
   }
   __syncthreads();
-  // The warps of a CTA start in lock step and every pair costs the same, so without a head start they reach the
-  // exchange (shared-memory bound) and the epilogue (MUFU bound) together and leave the FP32 pipe idle meanwhile.
-  // Warp w waits (w / 4) * stagger + (w % 4) * stagger / 4 cycles once: the three warps of a scheduler (w, w + 4,
-  // w + 8) and the four schedulers of the SM then sit in different phases of the loop.
-  if (stagger > 0) {
-    const long long t0 = clock64(), d = (long long)(warp >> 2) * stagger + (long long)(warp & 3) * (stagger >> 2);
-    while (clock64() - t0 < d) {}
-  }
+  const int group = warp & 3, rank = warp >> 2;
+  // RGBA rows leave through per-bin colour-map gathers and 4-byte stores; in lock step those stall the whole group and the
+  // rotation measured 7 % slower (467 vs 502 M frames/s at hop 512, 485 vs 522 at hop 256), so they keep free-running warps
+  constexpr bool kRotate = OUT != kOutRgba8;
 
   PairStep st;
   st.fpc = (int)g.frames_per_clip;
@@ -171,7 +202,6 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
   const int fpc = st.fpc;
   PairP cur;
   cur.fa = 2 * ((long long)blockIdx.x * NW + warp);
-  if (cur.fa >= g.total_frames) return;
   cur.clip = (int)(cur.fa / fpc);
   cur.t = (int)(cur.fa - (long long)cur.clip * fpc);
   cur.off = cur.clip * g.clip_stride + g.start0 + (long long)cur.t * HOP;
@@ -188,6 +218,8 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
     const float2* src = cur_fast ? reinterpret_cast<const float2*>(g.pcm + cur.off) + lane : idle_src;
     static_for<0, NLOAD>([&](auto mm) { constexpr int m = decltype(mm)::value; s[m] = ldg_nc_f2(src + 32 * m); });
   }
+  if (kRotate && cur.fa < g.total_frames)
+    for (int i = xp_lead(rank); i > 0; --i) xp_step_barrier(group, NW);
 
 #ifdef SG_XP_TRACE
   int trace_iter = 0;
@@ -196,7 +228,7 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
   unsigned dbg_epoch = 0;                       // this warp's pair counter
   unsigned* dbg_tags = dbg_warp_tags(warp);     // [0, 1024): exchange elements (writer lane, q); [1024, 2048): byte-stage entries
 #endif
-  while (true) {
+  while (cur.fa < g.total_frames) {   // a warp past total_frames has no pair and only runs its group's steps below
 #ifdef SG_DEBUG
     ++dbg_epoch;
     if (lane == 0) dbg_count_iteration();
@@ -245,6 +277,7 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
     //      unit (j, col) = [row 2j | row 2j+1].  Lane b stores its element k_a as one 8-byte half (STS.64, the 16
     //      lanes of a half-warp fill 8 whole units: conflict free); lane a then reads column a of a row pair with
     //      one LDS.128 -- rows b = 2j, 2j+1 hold q = bitrev4(j), bitrev4(j) + 16.
+    //      The step barrier between the stores (section A) and the loads (section B) also orders this warp's exchange.
     if constexpr (!(ABL & 1)) {
       float2* wre = reinterpret_cast<float2*>(xp) + ((lane >> 1) * kXpStride) * 2 + (lane & 1);
       float2* wim = wre + 16 * kXpStride * 2;
@@ -256,8 +289,11 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
         dbg_write(dbg_tags, lane * 32 + q, dbg_epoch);
 #endif
       });
-      asm volatile("bar.sync %0, 32;" ::"r"(warp + 1) : "memory");
-      XP_TRACE(2);
+    }
+    if constexpr (kRotate) xp_step_barrier(group, NW);   // ---- A | B
+    else asm volatile("bar.sync %0, 32;" ::"r"(warp + 1) : "memory");
+    XP_TRACE(2);
+    if constexpr (!(ABL & 1)) {
       const float4* rre = xp + lane;
       const float4* rim = rre + 16 * kXpStride;
       static_for<0, 16>([&](auto qq) {   // ascending q0: registers stored last are overwritten last
@@ -287,13 +323,6 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
 
     // a non-finite sample makes every Z of its frame non-finite: one test per frame. byte scale -> NaN -> byte 0
     const P2 poison = fma2(a[0].re, bc(0.f), mul2(a[0].im, bc(0.f)));   // 0 or NaN per frame
-
-    // ---- next pair: geometry now, its 40 loads interleaved with the untangle below (registers free up as the
-    //      untangle consumes Z), so HBM/L2 latency hides behind the untangle and the epilogue
-    const PairP nxt = pair_advance(cur, st);
-    const bool has_next = nxt.fa < g.total_frames;
-    const bool nxt_fast = has_next && pair_is_fast(g, nxt, st);
-    const float2* nsrc = nxt_fast ? reinterpret_cast<const float2*>(g.pcm + nxt.off) + lane : idle_src;
 
     // ---- untangle.  Z[1024 - k] for k = lane + 32 i is the partner lane's a[31 - i] (lane 0: its own a[32 - i]).
     //      First fetch every mirror IN PLACE (a[31 - i] <- partner's a[31 - i]; descending i keeps lane 0's own
@@ -343,6 +372,15 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
         }
       }
     });
+    if constexpr (kRotate) xp_step_barrier(group, NW);   // ---- B | C
+
+    // ---- next pair: geometry now, its 40 loads interleaved with the untangle below (registers free up as the
+    //      untangle consumes Z), so HBM/L2 latency hides behind the untangle and the epilogue
+    const PairP nxt = pair_advance(cur, st);
+    const bool has_next = nxt.fa < g.total_frames;
+    const bool nxt_fast = has_next && pair_is_fast(g, nxt, st);
+    const float2* nsrc = nxt_fast ? reinterpret_cast<const float2*>(g.pcm + nxt.off) + lane : idle_src;
+
     P2 pk[16], pm[16];
     static_for<0, 16>([&](auto ii) {
       constexpr int i = decltype(ii)::value;
@@ -433,15 +471,21 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
         if (has_b_out) { row_b[k] = bad_b ? z : vk.v.y; row_b[mk] = bad_b ? z : vm.v.y; }
       });
     }
-    __syncwarp();
     XP_TRACE(6);
+    if constexpr (kRotate) xp_step_barrier(group, NW);   // ---- C | A of the next pair (also orders the byte stage before the next exchange)
+    else __syncwarp();
 #ifdef SG_XP_TRACE
     ++trace_iter;
 #endif
-    if (!has_next) break;
     cur = nxt;
     cur_fast = nxt_fast;
   }
+  // barrier-only steps up to the group's count: the tail, or every step of a warp without pairs
+  if constexpr (kRotate)
+  for (long long i = xp_group_steps(g.total_frames, gridDim.x, NW, blockIdx.x, group) -
+                     xp_warp_steps(g.total_frames, gridDim.x, NW, blockIdx.x, warp);
+       i > 0; --i)
+    xp_step_barrier(group, NW);
 }
 
 }  // namespace sg

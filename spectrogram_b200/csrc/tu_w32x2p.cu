@@ -1,15 +1,7 @@
 // Translation unit: register-pipelined frame-pair kernel (n_fft 2048, hop 512).
-#include <cstdlib>
-
 #include "kernel_w32x2p.cuh"
 
 namespace sg {
-
-// head start between the warps of a CTA, in cycles (kernel_w32x2p.cuh); SG_XP_STAGGER overrides it for A/B runs
-static int xp_stagger() {
-  static const int v = [] { const char* e = getenv("SG_XP_STAGGER"); return e ? atoi(e) : 0; }();
-  return v;
-}
 
 template <int OUT, int NW, int HOPJ>
 static int launch_xp(const FrameGeom& g, const W32Plan& p, const Epilogue& ep, void* out, int sm_count, int device,
@@ -20,7 +12,7 @@ static int launch_xp(const FrameGeom& g, const W32Plan& p, const Epilogue& ep, v
   if (rc != cudaSuccess) return (int)rc;
   const long long pairs = (g.total_frames + 1) / 2;
   const int grid = (int)std::min<long long>((pairs + NW - 1) / NW, sm_count);
-  stft_w32x2p_kernel<OUT, NW, HOPJ><<<grid, NW * 32, smem, st>>>(g, p, ep, (T*)out, xp_stagger());
+  stft_w32x2p_kernel<OUT, NW, HOPJ><<<grid, NW * 32, smem, st>>>(g, p, ep, (T*)out);
   return (int)cudaGetLastError();
 }
 

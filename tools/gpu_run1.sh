@@ -1,15 +1,10 @@
 #!/bin/bash
-# round-2 GPU session 1: sanity, pipe microbenchmarks, phase timeline, stagger sweep, host-path ceiling
+# round-2 GPU session 1: sanity, pipe microbenchmarks, phase timeline, host-path ceiling
 cd "${GRAFT_REPO_ROOT:-.}"
 O=gpurun_out
 timeout 300 python -m pytest tests -m gpu -x -q 2>&1 | tail -3 > $O/r2_pytest1.log
 timeout 120 tools/microbench/xu_bench > $O/r2_xu_bench.txt 2>&1
-for s in 0 2000 6000; do timeout 60 tools/microbench/trace_bench $s > $O/r2_trace_$s.txt 2>&1; done
-: > $O/r2_stagger.txt
-for s in 0 300 1000 2000 4000 8000 16000; do
-  echo "stagger $s" >> $O/r2_stagger.txt
-  SG_XP_STAGGER=$s timeout 120 python tools/kbench.py 0 --clips 512 --steps 30 >> $O/r2_stagger.txt 2>&1
-done
+timeout 60 tools/microbench/trace_bench > $O/r2_trace.txt 2>&1
 timeout 120 python tools/host_path_ceiling.py > $O/r2_host_ceiling_n1.json 2>&1
 timeout 120 python tools/host_path_ceiling.py --bytes-per-sample 2 >> $O/r2_host_ceiling_n1.json 2>&1
 timeout 300 python bench.py --steps 20 --warmup 3 > $O/r2_bench1.json 2> $O/r2_bench1.err

@@ -20,7 +20,7 @@ void run(const Ctx& c, const char* what) {
   float best = 1e9f;
   for (int rep = 0; rep < 6; ++rep) {
     cudaEventRecord(e0);
-    stft_w32x2p_kernel<kOutU8, NW, 8, ABL><<<148, NW * 32, smem>>>(c.g, c.pl, c.ep, c.out, 0);
+    stft_w32x2p_kernel<kOutU8, NW, 8, ABL><<<148, NW * 32, smem>>>(c.g, c.pl, c.ep, c.out);
     cudaEventRecord(e1);
     if (cudaDeviceSynchronize() != cudaSuccess) { printf("ABL %d failed: %s\n", ABL, cudaGetErrorString(cudaGetLastError())); return; }
     float ms; cudaEventElapsedTime(&ms, e0, e1);

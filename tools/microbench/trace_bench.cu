@@ -4,7 +4,7 @@
 // Table values do not influence timing (no data-dependent branch), so the plan is filled with finite placeholders.
 // Build: nvcc -O3 -std=c++17 --expt-relaxed-constexpr -DSG_XP_TRACE -gencode arch=compute_100a,code=sm_100a \
 //        -I../../spectrogram_b200/csrc -o trace_bench trace_bench.cu
-// usage: trace_bench [stagger_cycles] [n_clips]
+// usage: trace_bench [n_clips]
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
@@ -14,8 +14,7 @@
 using namespace sg;
 
 int main(int argc, char** argv) {
-  const int stagger = argc > 1 ? atoi(argv[1]) : 0;
-  const int n_clips = argc > 2 ? atoi(argv[2]) : 256;
+  const int n_clips = argc > 1 ? atoi(argv[1]) : 256;
   constexpr int NW = 12, OUT = kOutU8, HOPJ = 8;
   const long long clip_len = 441000, fpc = 1 + (clip_len - 2048) / 512;
   float* pcm; cudaMalloc(&pcm, (size_t)n_clips * clip_len * 4);
@@ -41,18 +40,19 @@ int main(int argc, char** argv) {
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   for (int rep = 0; rep < 3; ++rep) {
     cudaEventRecord(e0);
-    stft_w32x2p_kernel<OUT, NW, HOPJ><<<148, NW * 32, smem>>>(g, pl, ep, out, stagger);
+    stft_w32x2p_kernel<OUT, NW, HOPJ><<<148, NW * 32, smem>>>(g, pl, ep, out);
     cudaEventRecord(e1);
     if (cudaDeviceSynchronize() != cudaSuccess) { printf("kernel failed: %s\n", cudaGetErrorString(cudaGetLastError())); return 1; }
     float ms; cudaEventElapsedTime(&ms, e0, e1);
-    printf("# stagger %d: %.4f ms, %.1f M frames/s (traced build)\n", stagger, ms, n_clips * fpc / ms * 1e-3);
+    printf("# %.4f ms, %.1f M frames/s (traced build)\n", ms, n_clips * fpc / ms * 1e-3);
   }
   std::vector<long long> t(tn);
   cudaMemcpy(t.data(), trace, tn * 8, cudaMemcpyDeviceToHost);
   long long t0 = -1;
   for (auto v : t) if (v && (t0 < 0 || v < t0)) t0 = v;
-  // phase p = [point p, point p+1): 0 window+pass1, 1 exchange stores+barrier, 2 exchange loads, 3 pass 2, 4 untangle
-  // (+ next pair's loads), 5 epilogue
+  // phase p = [point p, point p+1): 0 window+pass1, 1 exchange stores + the A|B step barrier, 2 exchange loads, 3 pass 2,
+  // 4 mirror shuffles + the B|C step barrier + untangle (+ next pair's loads), 5 epilogue; the C|A barrier falls between
+  // a pair's point 6 and the next pair's point 0 (kernel_w32x2p.cuh, rotation)
   printf("# warp iter start  window+p1 xstore xload pass2 untangle epilogue  total\n");
   for (int w = 0; w < NW; ++w)
     for (int it = 0; it < kXpTraceIters; ++it) {
