@@ -30,7 +30,9 @@
 namespace sg {
 
 // tools/microbench/trace_bench.cu builds this kernel with SG_XP_TRACE: lane 0 of every warp of CTA 0 records clock64 at
-// the phase boundaries of its first kXpTraceIters pairs (the product build compiles the hooks away)
+// the top of each of its first kXpTraceIters pairs (point 0) and just before and just after each of the pair's three group
+// barriers (points 1 / 2: A | B, 3 / 4: B | C, 5 / 6: C | A), so each section's busy time and each barrier's wait are
+// separable (the product build compiles the hooks away)
 #ifdef SG_XP_TRACE
 constexpr int kXpTraceIters = 40, kXpTracePoints = 8;
 __device__ long long* g_xp_trace;
@@ -61,9 +63,11 @@ struct XpShape {
   static constexpr int kMaxRegs = NW <= 8 ? 255 : (65536 / (NW * 32)) / 8 * 8;
 };
 
-// Rotation.  A pair runs as three sections of similar FP32-pipe demand but different non-FMA content:
+// Rotation.  A pair runs as three sections of different non-FMA content (the cuts between them: xp_cuts below).  Round 3's
+// placement, which every output but 12-warp bytes keeps:
 //   A  window + pass 1 + exchange stores         B  exchange loads + pass 2 + mirror shuffles / selects
 //   C  untangle with the next pair's loads + epilogue
+// 12-warp bytes move the exchange stores into B and the byte de-interleave (row stores) into the next pair's A.
 // The warps of one scheduler (w, w + 4, w + 8: a rotation group) would otherwise reach the exchange, the shuffles and the
 // MUFU epilogue together and leave the FP32 pipe idle meanwhile.  Instead the group runs in steps separated by one group
 // barrier (ID 1 + group, NW / 4 warps): at step s, rank k (= w / 4) runs section (s + k) mod 3, so the ranks always sit in
@@ -94,6 +98,24 @@ __host__ __device__ inline long long xp_group_steps(long long total_frames, int 
 }
 __device__ __forceinline__ void xp_step_barrier(int group, int nw) {
   asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "r"(nw / 4 * 32) : "memory");
+}
+
+// Where the three group barriers of a pair sit (a pair stays three sections whatever the cuts, so the step counts above
+// do not depend on them), packed as xp_cut(ab, bc, ca):
+//   ab  A | B   0: before the exchange loads                1: after them          2: before the exchange stores
+//   bc  B | C   0: after pass-2 stage 9 (stage 10 in C)     1: after stage 10     2: after the mirror shuffles and selects
+//   ca  C | A   0: before the byte de-interleave (u8 only: its loads, PRMTs and row stores open the next section A)
+//               1: at the end of the pair
+// A cut away from a point where its barrier also ordered the warp's own shared-memory hand-off leaves a __syncwarp()
+// there: exchange stores -> exchange loads, and byte stage -> the next pair's exchange stores.
+// tools/microbench/rotation_cut_bench.cu times every placement (profiles/r04_cut_sweep.txt).  Byte rows with 12 warps
+// take the exchange stores into B and the byte de-interleave into the next A: hop 512 (the headline) 636 -> 660 M frames/s
+// with B | C where round 3 put it, hop 256 640 -> 651 M with B | C after stage 9.  Every other instantiation measured no
+// gain from moving a cut and keeps round 3's.
+__host__ __device__ constexpr int xp_cut(int ab, int bc, int ca) { return ab * 100 + bc * 10 + ca; }
+template <int OUT, int NW, int HOPJ>
+constexpr int xp_cuts() {
+  return OUT != kOutU8 || NW != 12 ? xp_cut(0, 2, 1) : HOPJ == 8 ? xp_cut(2, 2, 0) : xp_cut(2, 0, 0);
 }
 
 // stage U (1..5) of pass 2: butterflies (i0, i0 + half), twiddle W_{2 half}^p * base
@@ -151,11 +173,16 @@ __device__ __forceinline__ bool pair_is_fast(const FrameGeom& g, const PairP& p,
 // wrong, the time saved is that component's marginal cost under the real contention: 1 exchange, 2 mirror shuffles,
 // 4 MUFU/F2IP, 8 next-pair loads, 16 byte stage + row stores, 32 window table reads, 64 lane-0 selects (128: the
 // selects as PRMT instead of FSEL; 256: the mirrors through shared memory instead of shuffles)
-template <int OUT, int NW, int HOPJ = 8, int ABL = 0>   // hop = 64 * HOPJ samples: frame B's element j is element j + HOPJ of the lane
+// CUT moves the rotation's barriers (xp_cut above); tools/microbench/rotation_cut_bench.cu sets it, product launches take
+// the default
+template <int OUT, int NW, int HOPJ = 8, int ABL = 0,   // hop = 64 * HOPJ samples: frame B's element j is element j + HOPJ of the lane
+          int CUT = xp_cuts<OUT, NW, HOPJ>()>
 __global__ void __launch_bounds__(NW * 32, 1) __maxnreg__(XpShape<NW>::kMaxRegs)
 stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::type* __restrict__ out) {
   using T = typename OutElem<OUT>::type;
   constexpr int HOP = 64 * HOPJ, NLOAD = 32 + HOPJ, kLoadSteps = xp_load_steps<OUT, HOPJ>();
+  constexpr int kCutAB = CUT / 100, kCutBC = CUT / 10 % 10, kCutCA = CUT % 10;
+  static_assert(kCutAB <= 2 && kCutBC <= 2 && kCutCA <= 1 && (kCutCA == 1 || OUT == kOutU8), "no such cut");
   extern __shared__ float4 smem_raw[];
   float4* s_win4 = smem_raw;                                           // [16][32] (w2[l+32j], w2[l+32(j+16)])
   float2* s_twb = reinterpret_cast<float2*>(s_win4 + 16 * 32);         // [5][32]  W_{32*2^u}^lane
@@ -271,13 +298,13 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
     dit2_stage_const<3>(a);
     dit2_stage_const<4>(a);
     dit2_stage_const<5>(a);
-    XP_TRACE(1);
 
     // ---- exchange (32x32 transpose).  Each plane (re, im) keeps rows 2j and 2j+1 interleaved in 16-byte units:
     //      unit (j, col) = [row 2j | row 2j+1].  Lane b stores its element k_a as one 8-byte half (STS.64, the 16
     //      lanes of a half-warp fill 8 whole units: conflict free); lane a then reads column a of a row pair with
     //      one LDS.128 -- rows b = 2j, 2j+1 hold q = bitrev4(j), bitrev4(j) + 16.
-    //      The step barrier between the stores (section A) and the loads (section B) also orders this warp's exchange.
+    //      The A | B barrier, when it falls between the stores and the loads, also orders this warp's exchange.
+    if constexpr (kRotate && kCutAB == 2) { XP_TRACE(1); xp_step_barrier(group, NW); XP_TRACE(2); }   // ---- A | B
     if constexpr (!(ABL & 1)) {
       float2* wre = reinterpret_cast<float2*>(xp) + ((lane >> 1) * kXpStride) * 2 + (lane & 1);
       float2* wim = wre + 16 * kXpStride * 2;
@@ -290,9 +317,9 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
 #endif
       });
     }
-    if constexpr (kRotate) xp_step_barrier(group, NW);   // ---- A | B
-    else asm volatile("bar.sync %0, 32;" ::"r"(warp + 1) : "memory");
-    XP_TRACE(2);
+    if constexpr (!kRotate) asm volatile("bar.sync %0, 32;" ::"r"(warp + 1) : "memory");
+    else if constexpr (kCutAB == 0) { XP_TRACE(1); xp_step_barrier(group, NW); XP_TRACE(2); }   // ---- A | B
+    else __syncwarp();
     if constexpr (!(ABL & 1)) {
       const float4* rre = xp + lane;
       const float4* rim = rre + 16 * kXpStride;
@@ -310,16 +337,17 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
       });
       __syncwarp();
     }
-    XP_TRACE(3);
+    if constexpr (kRotate && kCutAB == 1) { XP_TRACE(1); xp_step_barrier(group, NW); XP_TRACE(2); }   // ---- A | B
 
     // ---- pass 2: stages 6-10, twiddles from the five per-lane bases
     dit2_stage_gen<1>(a, s_twb[0 * 32 + lane]);
     dit2_stage_gen<2>(a, s_twb[1 * 32 + lane]);
     dit2_stage_gen<3>(a, s_twb[2 * 32 + lane]);
     dit2_stage_gen<4>(a, s_twb[3 * 32 + lane]);
+    if constexpr (kRotate && kCutBC == 0) { XP_TRACE(3); xp_step_barrier(group, NW); XP_TRACE(4); }   // ---- B | C
     dit2_stage_gen<5>(a, s_twb[4 * 32 + lane]);
     // now a[i] = Z[lane + 32 i] of both frames
-    XP_TRACE(4);
+    if constexpr (kRotate && kCutBC == 1) { XP_TRACE(3); xp_step_barrier(group, NW); XP_TRACE(4); }   // ---- B | C
 
     // a non-finite sample makes every Z of its frame non-finite: one test per frame. byte scale -> NaN -> byte 0
     const P2 poison = fma2(a[0].re, bc(0.f), mul2(a[0].im, bc(0.f)));   // 0 or NaN per frame
@@ -372,7 +400,7 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
         }
       }
     });
-    if constexpr (kRotate) xp_step_barrier(group, NW);   // ---- B | C
+    if constexpr (kRotate && kCutBC == 2) { XP_TRACE(3); xp_step_barrier(group, NW); XP_TRACE(4); }   // ---- B | C
 
     // ---- next pair: geometry now, its 40 loads interleaved with the untangle below (registers free up as the
     //      untangle consumes Z), so HBM/L2 latency hides behind the untangle and the epilogue
@@ -407,7 +435,6 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
         });
       }
     });
-    XP_TRACE(5);
     // ---- epilogue
     const bool has_b_out = cur.fa + 1 < g.total_frames;
     T* __restrict__ row_a = out + cur.fa * (long long)kW32M;
@@ -437,8 +464,11 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
           if (has_b_out) { row_b[k] = __ldg(ep.lut + kb); row_b[mk] = __ldg(ep.lut + mb); }
         }
       });
+      if constexpr (OUT == kOutU8 && !(ABL & 16)) __syncwarp();
+      if constexpr (OUT == kOutU8 && kCutCA == 0) {   // ---- C | A of the next pair
+        XP_TRACE(5); xp_step_barrier(group, NW); XP_TRACE(6);
+      }
       if constexpr (OUT == kOutU8 && !(ABL & 16)) {
-        __syncwarp();
         // de-interleave the (A,B) byte pairs: 8 bins per lane per round, 8-byte coalesced row stores
         const uint4* s16 = reinterpret_cast<const uint4*>(sb16);
         uint2* ra = reinterpret_cast<uint2*>(row_a);
@@ -471,8 +501,8 @@ stft_w32x2p_kernel(FrameGeom g, W32Plan pl, Epilogue ep, typename OutElem<OUT>::
         if (has_b_out) { row_b[k] = bad_b ? z : vk.v.y; row_b[mk] = bad_b ? z : vm.v.y; }
       });
     }
-    XP_TRACE(6);
-    if constexpr (kRotate) xp_step_barrier(group, NW);   // ---- C | A of the next pair (also orders the byte stage before the next exchange)
+    // ---- C | A of the next pair (or, where it does not fall here, the byte stage before the next exchange)
+    if constexpr (kRotate && kCutCA == 1) { XP_TRACE(5); xp_step_barrier(group, NW); XP_TRACE(6); }
     else __syncwarp();
 #ifdef SG_XP_TRACE
     ++trace_iter;
